@@ -295,9 +295,11 @@ NN_API int nn_edge_geom_bwd(const float* x_bar, int32_t n_slots, const float* un
 /* image of message_edgepart.weight [128, 20] for the tensor-core message kernels (2 * 4096 floats). */
 #define NN_WE_IMAGE_FLOATS (2 * 128 * 32)
 NN_API int nn_message_prepare_b(const float* We, float* image, void* stream);
-/* m_p = (We rbf_p) * mn_i * mn_j, models/newtonnet.py:210-211. */
+/* m_p = (We rbf_p) * mn_i * mn_j, models/newtonnet.py:210-211, for the pairs p < status[NN_ST_N_PAIRS] (rows past the
+ * count are not written).  Tensor-core backend (nn_get_gemm_backend() >= 1) with We_img != NULL: the persistent tcgen05
+ * kernel (3xTF32, We_img from nn_message_prepare_b) that nn_eval runs; otherwise the fp32 SIMT kernel, which needs Wet. */
 NN_API int nn_edge_message_fwd(const nn_nbr* nl, const float* rbf, const float* mn, const float* Wet,
-                        float* msg, void* stream);
+                               const float* We_img, float* msg, void* stream);
 /* a_out = a + sum_e m ; f_out = f + sum_e (e1 u + e2 * f_j), models/newtonnet.py:213-227. */
 NN_API int nn_node_aggregate_fwd(const nn_nbr* nl, const float* msg, const float* e1, const float* e2,
                           const float* unit, const float* a_in, const float* f_in, float* a_out,

@@ -137,7 +137,7 @@ SYMBOLS = {
     'nn_edge_geom_fwd': (C.c_int, [_fp, _fp, C.c_float, _fp, C.c_int32, _fp, _fp, _fp, _fp, _fp]),
     'nn_edge_geom_bwd': (C.c_int, [_fp, C.c_int32, _fp, _fp, _fp, C.c_float, _fp, C.c_int32, _fp, _fp]),
     'nn_message_prepare_b': (C.c_int, [_fp, _fp, _fp]),
-    'nn_edge_message_fwd': (C.c_int, [C.POINTER(Nbr), _fp, _fp, _fp, _fp, _fp]),
+    'nn_edge_message_fwd': (C.c_int, [C.POINTER(Nbr), _fp, _fp, _fp, _fp, _fp, _fp]),
     'nn_node_aggregate_fwd': (C.c_int, [C.POINTER(Nbr), _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, C.c_int32, _fp]),
     'nn_equiv_update_fwd': (C.c_int, [_fp, _fp, _fp, _fp, C.c_int32, _fp]),
     'nn_energy_head_fwd': (C.c_int, [_fp, _fp, _fp, _fp, _fp, _fp, _fp, C.c_int32, C.c_int32, _fp, _fp, _fp]),

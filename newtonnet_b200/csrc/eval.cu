@@ -24,6 +24,8 @@ int nn_layer_norm_fwd_launch(float* a_io, const float* gamma, const float* beta,
 int nn_layer_norm_bwd_launch(float* abar_io, const float* gamma, const float* xhat, const float* rstd, int n_rows, cudaStream_t s);
 int nn_direct_force_launch(const float* h, const float* f, const float* scale, const int64_t* z, int n_rows, float* out, cudaStream_t s);
 int nn_message_fwd_tc(const nn_nbr* nl, const float* rbf, const float* mn, const float* We_img, float* msg, cudaStream_t s);
+int nn_edge_message_fwd_launch(const nn_nbr* nl, const float* rbf, const float* mn, const float* Wet, float* msg,
+                               cudaStream_t s);
 int nn_message_bwd_tc(const nn_nbr* nl, const float* abar, const float* mn, const float* rbf, const float* drbf,
                       const float* We_img, float* mbar_io, float* x_part, cudaStream_t s);
 int nn_node_aggregate_bwd_launch(const nn_nbr* nl, int n_rows, const float* t, const float* mn, const float* e2,
@@ -389,8 +391,7 @@ int run_phase(EvalCtx& c, int phase, int l) {
         const float* f_in = first ? nullptr : w.layer[l - 1].f_out;
         {
             ProfScope ps(NN_STAGE_MESSAGE, s);
-            if (g_backend >= 1 && lw.We_img) NN_TRY(nn_message_fwd_tc(nl, w.rbf, b.mn, lw.We_img, b.msg, s));
-            else NN_TRY(nn_edge_message_fwd(nl, w.rbf, b.mn, lw.Wet, b.msg, s));
+            NN_TRY(nn_edge_message_fwd(nl, w.rbf, b.mn, lw.Wet, lw.We_img, b.msg, s));
         }
         // layer 0: force_node == 0, so equiv_message2 contributes exactly nothing; other layers: both MLPs in one dual launch
         if (first || !g.mlp_fwd_dual(b.msg, lw.U1, b.q1, lw.U2, b.e1, lw.V1, b.q2, lw.V2, b.e2, P, np_dev)) {
@@ -529,6 +530,14 @@ extern "C" NN_API int nn_pair_gather_bwd(const nn_nbr* nl, const float* dfb, con
                                          float* e2bar, float* ubar, void* stream) {
     NN_REQUIRE(nl && dfb && unit && e1_io && ubar && (f_in == nullptr || e2bar != nullptr), "null pointer");
     return nn_pair_bwd_gather_launch(nl, dfb, f_in, unit, e1_io, e2bar, ubar, f_in == nullptr, (cudaStream_t)stream);
+}
+
+extern "C" NN_API int nn_edge_message_fwd(const nn_nbr* nl, const float* rbf, const float* mn, const float* Wet, const float* We_img,
+                                          float* msg, void* stream) {
+    NN_REQUIRE(nl && rbf && mn && msg && (Wet || We_img), "null pointer");
+    if (g_backend >= 1 && We_img) return nn_message_fwd_tc(nl, rbf, mn, We_img, msg, (cudaStream_t)stream);
+    NN_REQUIRE(Wet != nullptr, "the SIMT backend needs Wet");
+    return nn_edge_message_fwd_launch(nl, rbf, mn, Wet, msg, (cudaStream_t)stream);
 }
 
 extern "C" NN_API int nn_edge_message_bwd(const nn_nbr* nl, const float* abar, const float* mn, const float* rbf, const float* drbf,

@@ -720,12 +720,13 @@ extern "C" int nn_edge_geom_bwd(const float* x_bar, int32_t n_slots, const float
     return 0;
 }
 
-extern "C" int nn_edge_message_fwd(const nn_nbr* nl, const float* rbf, const float* mn, const float* Wet, float* msg,
-                                   void* stream) {
+// SIMT twin of the tensor-core message kernel; the public nn_edge_message_fwd (eval.cu) picks between them
+int nn_edge_message_fwd_launch(const nn_nbr* nl, const float* rbf, const float* mn, const float* Wet, float* msg,
+                               cudaStream_t s) {
     if (nl->cap_pairs <= 0) return 0;
-    k_edge_message_fwd<<<grid_for_rows(nl->n_atoms), kThreads, 0, (cudaStream_t)stream>>>(
+    k_edge_message_fwd<<<grid_for_rows(nl->n_atoms), kThreads, 0, s>>>(
         nl->pair_ptr, nl->pair_j, nl->n_atoms, nl->cap_pairs, rbf, mn, Wet, msg); NN_LAUNCHED(1);
-    NN_CHECK_LAUNCH("nn_edge_message_fwd");
+    NN_CHECK_LAUNCH("message_fwd(simt)");
     return 0;
 }
 

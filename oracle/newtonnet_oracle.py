@@ -390,10 +390,14 @@ def forward_analytic(sd, z, pos, cell, batch, dtype=torch.float64, cutoff=CUTOFF
         h = cell[batch[pi]]
         nimg = torch.round(torch.linalg.solve(h.transpose(1, 2), dpos))
         M = M - torch.bmm(h.transpose(1, 2), G.unsqueeze(2)) * nimg.unsqueeze(1)
+    M_pair = M
     M = _segment_sum(M, batch[pi], n_sys)
     g_D = 0.5 * (M + M.transpose(1, 2))
+    # per-pair terms too (pairs [2,P] = (i<j), G = dE/d disp, M before the per-system sum): what one atom or one pair
+    # contributes to the virial, for tests that must notice an atom dropped from or counted twice in a sum
     out = {'energy': energy.numpy(), 'forces': (-g_pos).numpy(), 'virial': (-g_D).numpy(),
-           'atom_node': a.numpy(), 'force_node': f.numpy()}
+           'atom_node': a.numpy(), 'force_node': f.numpy(), 'pairs': torch.stack([pi, pj]).numpy(),
+           'G': G.numpy(), 'M': M_pair.numpy()}
     if bool((cell != 0).any()):
         out['stress'] = (g_D / torch.linalg.det(cell).view(-1, 1, 1)).numpy()
     return out
