@@ -474,6 +474,23 @@ NN_API int nn_md_finish(int32_t n_systems, const int32_t* sys_ptr, double* v, co
                         double dt, const float* energy, double* log, int32_t log_cap, int64_t* step_ctr,
                         const int32_t* nbr_status, int32_t* sticky, uint32_t* ticket, void* stream);
 
+/* ---- Hessian in blocks of rows (newtonnet_b200/hessian.py; reference models/output.py:141-152 batches rows with vmap) ----
+ * A pass puts k copies of frames of n_slot atoms into one batch (copy c = system c) and differentiates <seed, pos_grad>
+ * once: copy c's block of that gradient is row plan[pass][c].row of its frame's Hessian.
+ * plan: [n_pass, k, 3] int32 {frame, local row in [0, 3 n_slot) or -1 for a padding job, output row};
+ * frame_ptr: [n_frames + 1] first atom of each frame of the input batch; every planned frame has n_slot atoms.
+ * *pass_ctr: index of the pass both calls work on (device memory: a captured pass replays without host traffic).
+ * expand: z_rep [k n_slot], pos_rep [k n_slot, 3], cell_rep [k,3,3], batch_rep [k n_slot] (= copy index), seed [k n_slot, 3]
+ *         (one-hot at the job's row in its copy's block; all zero for a padding job). */
+NN_API int nn_hessian_expand(const int32_t* plan, const int32_t* pass_ctr, int32_t k, int32_t n_slot, const int64_t* z,
+                             const float* pos, const float* cell, const int32_t* frame_ptr, int64_t* z_rep, float* pos_rep,
+                             float* cell_rep, int64_t* batch_rep, float* seed, void* stream);
+/* H[out, :] for each real job of the pass: columns 3 frame_ptr[f] .. 3 frame_ptr[f+1] from copy c of grad_rep [k n_slot, 3],
+ * all other n_cols columns 0 (each element written once, no atomics); padding jobs write nothing.  Then advances
+ * *pass_ctr by one (ticket: one zero-initialised uint32, returned to 0 by the call). */
+NN_API int nn_hessian_scatter(const int32_t* plan, int32_t* pass_ctr, int32_t k, int32_t n_slot, const int32_t* frame_ptr,
+                              const float* grad_rep, float* H, int64_t n_cols, uint32_t* ticket, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

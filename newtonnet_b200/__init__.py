@@ -7,3 +7,4 @@ used for device memory, streams and torch.distributed only.  No CPU fallback.
 __version__ = '0.1.0'
 
 from newtonnet_b200.models.newtonnet import NewtonNet  # noqa: F401
+from newtonnet_b200.hessian import hessian  # noqa: F401,E402  (the function; the module is newtonnet_b200.hessian)

@@ -142,6 +142,8 @@ SYMBOLS = {
     'nn_equiv_update_fwd': (C.c_int, [_fp, _fp, _fp, _fp, C.c_int32, _fp]),
     'nn_energy_head_fwd': (C.c_int, [_fp, _fp, _fp, _fp, _fp, _fp, _fp, C.c_int32, C.c_int32, _fp, _fp, _fp]),
     'nn_force_virial_reduce': (C.c_int, [C.POINTER(Nbr), _fp, _fp, _fp, _fp, _fp, _fp]),
+    'nn_hessian_expand': (C.c_int, [_fp, _fp, C.c_int32, C.c_int32, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp]),
+    'nn_hessian_scatter': (C.c_int, [_fp, _fp, C.c_int32, C.c_int32, _fp, _fp, _fp, C.c_int64, _fp, _fp]),
 }
 
 _lib = None

@@ -751,13 +751,27 @@ def _table(emb, onehot):
     return torch.mv(onehot[:, :w.shape[0]] if w.shape[0] <= onehot.shape[1] else onehot, w).unsqueeze(1)
 
 
-def differentiable_forward(model, z, pos, cell, batch, static_nl=None):
+def hessian_rows(pos_grad, pos):
+    """d pos_grad / d pos [N,3,N,3] with one reverse pass per row of the 3N x 3N matrix (reference models/output.py:141-152
+    batches the same rows with vmap).  pos_grad must carry a graph to pos (create_graph=True).  Every row's pass walks the
+    whole batch: 3N passes over N atoms.  The rows themselves carry no graph: a third derivative through the fused SiLU and
+    radial-basis kernels is not implemented (SiluB.backward, _rbf_raw)."""
+    flat = pos_grad.reshape(-1)
+    with _skip_weight_grads():
+        rows = [torch.autograd.grad(flat[r], pos, retain_graph=True, create_graph=False)[0] for r in range(flat.numel())]
+    N = pos.shape[0]
+    return torch.stack(rows).reshape(N, 3, N, 3)
+
+
+def differentiable_forward(model, z, pos, cell, batch, static_nl=None, properties=None):
     """NewtonNet.forward with create_graph semantics (reference models/newtonnet.py:74-104 in train mode).
     static_nl: a NeighborList of fixed capacity already rebuilt for `pos` on the current stream -> the whole forward
-    has static shapes and no host synchronisation (GraphedTrainingStep)."""
+    has static shapes and no host synchronisation (GraphedTrainingStep).
+    properties: the outputs to form (default: model.output_properties; heads are looked up in the model's own list)."""
     from newtonnet_b200.engine import get_engine
     from newtonnet_b200.models.output import CustomOutputSet
-    props = list(model.output_properties)
+    own = list(model.output_properties)
+    props = own if properties is None else list(properties)
     if 'energy' not in props:
         raise RuntimeError("output_properties must contain 'energy'")
     for key in props:
@@ -825,7 +839,7 @@ def differentiable_forward(model, z, pos, cell, batch, static_nl=None):
         a = a + SumMulC.apply(f.view(N, 3, F), g)
         if layer.layer_norm is not None:
             a = Fn.layer_norm(a, (F,), layer.layer_norm.weight, layer.layer_norm.bias, layer.layer_norm.eps)
-    k = props.index('energy')
+    k = own.index('energy')
     head, scaler = model.output_layers[k].layers, model.scalers[k]
     h = silu(linear(a, head[0].weight, head[0].bias))
     h = silu(linear(h, head[2].weight, head[2].bias))
@@ -838,25 +852,25 @@ def differentiable_forward(model, z, pos, cell, batch, static_nl=None):
         if key == 'energy':
             out.energy = energy
         elif key == 'direct_force':
-            kd = props.index(key)
+            kd = own.index(key)
             dl, ds = model.output_layers[kd].layers, model.scalers[kd]
             hd = silu(linear(a, dl[0].weight, dl[0].bias))
             hd = linear(silu(linear(hd, dl[2].weight, dl[2].bias)), dl[4].weight, dl[4].bias)
             out.direct_force = RowDot.apply(f.view(N, 3, F), hd) * _table(ds.scale, onehot)
         elif key == 'hessian':
-            # reference models/output.py:141-152 (vmap over unit vectors): one reverse pass per row of the 3N x 3N matrix
+            # reference models/output.py:141-152 (vmap over unit vectors)
             if not hasattr(out, 'pos_grad') or not out.pos_grad.requires_grad:
                 raise RuntimeError("'hessian' needs 'gradient_force' evaluated before it with create_graph=True "
                                    "(MLAseCalculator sets this, reference utils/ase_interface.py:125-128)")
-            flat = out.pos_grad.reshape(-1)
-            keep = bool(model.output_layers[props.index(key)].create_graph)
-            with _skip_weight_grads():
-                rows = [torch.autograd.grad(flat[r], pos, retain_graph=True, create_graph=False)[0] for r in range(flat.numel())]
-            out.hessian = torch.stack(rows).reshape(N, 3, N, 3)
-            if not keep:
-                out.hessian = out.hessian.detach()
+            # training with create_graph heads (NewtonNet.train()) keeps the per-row loop; otherwise - MLAseCalculator, which
+            # sets create_graph on every derivative head as the reference does, evaluates in eval mode - rows in batched blocks
+            if model.training and bool(model.output_layers[own.index(key)].create_graph):
+                out.hessian = hessian_rows(out.pos_grad, pos)
+            else:
+                from newtonnet_b200.hessian import hessian_blocks     # rows in batched blocks (newtonnet_b200/hessian.py)
+                out.hessian = hessian_blocks(model, z, pos.detach(), cell, batch)
         else:
-            create = bool(model.output_layers[props.index(key)].create_graph) or 'hessian' in props
+            create = bool(model.output_layers[own.index(key)].create_graph) or 'hessian' in props
             with _skip_weight_grads():              # only d/d pos is asked for: no X^T dY products in this sweep
                 out.pos_grad, = torch.autograd.grad(energy, pos, torch.ones_like(energy), create_graph=create,
                                                     retain_graph=create)
