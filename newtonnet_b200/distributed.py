@@ -22,6 +22,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib as L
+from .engine import NeighborList, capture, count_edges, edge_capacity, edges_needed, eval_args, get_engine, stream
 
 GRIDS = {1: (1, 1, 1), 2: (2, 1, 1), 3: (3, 1, 1), 4: (2, 2, 1), 6: (3, 2, 1), 8: (2, 2, 2)}
 
@@ -133,7 +134,7 @@ class HaloExchange:
             return out
         if rows.is_cuda:
             L.check(L.load().nn_halo_pack(rows.data_ptr(), self.send_index.data_ptr(), self.n_send, width,
-                                          out.data_ptr(), torch.cuda.current_stream().cuda_stream), 'nn_halo_pack')
+                                          out.data_ptr(), stream()), 'nn_halo_pack')
         else:   # host tensors: used only by the gloo tests of the plan / exchange logic
             torch.index_select(rows, 0, self.send_index.long(), out=out)
         return out
@@ -270,10 +271,11 @@ class _PeerStep:
     """One decomposed evaluation over static buffers: launched eagerly the first time, then captured and replayed
     as ONE CUDA graph (two streams: halo exchanges off the critical path run on the side stream)."""
 
+    HEADROOM = (1.08, 64)          # both capacities: factor and slack over the trial fill's edge and pair counts
+
     def __init__(self, dd, z, pos, cell3, want_virial, reuse=None):
         """reuse: the step object of the previous plan of the same box - its arena (peer mappings) and its neighbour-list
         capacities are taken over when they fit, and the first call is captured right away (every kernel has run before)."""
-        from newtonnet_b200.engine import NeighborList, get_engine
         self.dd = dd
         dev = pos.device
         self.device = dev
@@ -325,54 +327,40 @@ class _PeerStep:
         self.graph = None
         self.calls = 0
         self.stale = False
-        self._NeighborList = NeighborList
         self.nl = None
         if fits and reuse.nl is not None:
             # capacities of the previous plan, scaled by the change of the owned count, plus headroom (an overflow is caught by
             # the status words like any other)
             g = max(1.0, self.n_owned / max(reuse.n_owned, 1)) * 1.02
-            self._size_neighbor_list(caps=(int(reuse.nl.cap_edges * g) + 64, int(reuse.nl.cap_pairs * g) + 64))
+            self._bind_list(edge_capacity(reuse.nl.cap_edges, g, 64), int(reuse.nl.cap_pairs * g) + 64)
             self.calls = 1               # no eager first step: capture immediately
         else:
             self._size_neighbor_list()
 
     # ---- capacities
     def _new_list(self, cap_edges, cap_pairs):
-        nl = self._NeighborList(self.engine, self.pos_l, self.cell_in, self.batch_l, cap_edges=cap_edges, cap_pairs=cap_pairs)
-        nl.struct.n_owned = self.n_owned
-        return nl
+        return NeighborList(self.engine, self.pos_l, self.cell_in, self.batch_l, cap_edges, cap_pairs, self.n_owned)
 
-    def _size_neighbor_list(self, needed=None, caps=None):
+    def _size_neighbor_list(self, needed=0):
         """Probe: count (-> directed edges of the owned rows), then a trial fill with room for one pair per edge (ghost rows
-        are empty, so an owned-ghost pair has a single directed edge and P lies between E / 2 and E) -> final capacities.
-        caps = (cap_edges, cap_pairs): take these instead of probing."""
-        s = torch.cuda.current_stream().cuda_stream
-        if caps is not None:
-            self.nl = self._new_list(caps[0] + caps[0] % 2, caps[1])
-            self._bind_eval()
-            return
-        probe = self._new_list(0, 0)
-        L.check(self.lib.nn_nbr_count(C.byref(probe.struct), self.pack.cutoff, s), 'nn_nbr_count')
-        n_edges = max(probe.check()[L.ST_N_EDGES], int(needed or 0))
+        are empty, so an owned-ghost pair has a single directed edge and P lies between E / 2 and E) -> final capacities."""
+        probe = count_edges(self.engine, self.pos_l, self.cell_in, self.batch_l, self.pack.cutoff, self.n_owned)
+        n_edges = max(probe.n_edges, needed)
         probe = self._new_list(n_edges + 2, n_edges + 2)
-        L.check(self.lib.nn_nbr_count(C.byref(probe.struct), self.pack.cutoff, s), 'nn_nbr_count')
-        L.check(self.lib.nn_nbr_fill(C.byref(probe.struct), self.pack.cutoff, s), 'nn_nbr_fill')
+        probe.rebuild(self.pack.cutoff)
         st = probe.check()
-        cap = int(st[L.ST_N_EDGES] * 1.08) + 64
-        self.nl = self._new_list(cap + cap % 2, int(st[L.ST_N_PAIRS] * 1.08) + 64)
         del probe
-        self._bind_eval()
+        factor, slack = self.HEADROOM
+        self._bind_list(edge_capacity(st[L.ST_N_EDGES], factor, slack), int(st[L.ST_N_PAIRS] * factor) + slack)
 
-    def _bind_eval(self):
+    def _bind_list(self, cap_edges, cap_pairs):
+        self.nl = self._new_list(cap_edges, cap_pairs)
         nbytes = self.lib.nn_eval_workspace_bytes(self.n_local, 1, self.nl.cap_pairs, self.pack.n_layers, 1)
         self.ws = torch.empty(int(nbytes) + 256, dtype=torch.uint8, device=self.device)
-        a = L.EvalArgs()
-        a.nbr, a.w, a.z = C.pointer(self.nl.struct), C.pointer(self.pack.struct), self.z_l.data_ptr()
-        a.want_forces, a.want_virial, a.n_owned = 1, int(self.want_virial), self.n_owned
-        a.energy, a.forces = self.energy.data_ptr(), self.forces_l.data_ptr()
-        a.virial, a.stress = (self.virial.data_ptr(), self.stress.data_ptr()) if self.want_virial else (None, None)
-        a.workspace, a.workspace_bytes = self.ws.data_ptr(), self.ws.numel()
-        self.args = a
+        out = {'energy': self.energy, 'forces': self.forces_l}
+        if self.want_virial:
+            out.update(virial=self.virial, stress=self.stress)
+        self.args = eval_args(self.nl, self.pack, self.z_l, out, self.ws, True, self.want_virial, self.n_owned)
         self.graph = None
         self.calls = 0
 
@@ -409,8 +397,7 @@ class _PeerStep:
         L.check(lib.nn_dd_begin(comm, self.pos_in.data_ptr(), self.pos_ref.data_ptr(), self.cell_in.data_ptr(),
                                 self.cell_ref.data_ptr(), self.z_in.data_ptr(), self.l2g.data_ptr(), self.n_local,
                                 self.dd.skin, self.pos_l.data_ptr(), self.z_l.data_ptr(), s), 'nn_dd_begin')
-        L.check(lib.nn_nbr_count(C.byref(self.nl.struct), self.pack.cutoff, s), 'nn_nbr_count')
-        L.check(lib.nn_nbr_fill(C.byref(self.nl.struct), self.pack.cutoff, s), 'nn_nbr_fill')
+        self.nl.rebuild(self.pack.cutoff)
         phase(L.PH_BEGIN)
         pending = False
         for l in range(nL):
@@ -451,11 +438,19 @@ class _PeerStep:
             self._launch()
             return
         if self.graph is None:
-            torch.cuda.synchronize(self.device)
-            self.graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(self.graph):
-                self._launch()
+            self.graph, _, _ = capture(self._launch, self.device)
         self.graph.replay()
+
+    def status(self):
+        """Status words of the last step (one small D2H copy, synchronises); raises when a peer timed out or a rank's
+        inputs broke its neighbour list."""
+        st = self.out_status.cpu().tolist()
+        if st[L.DD_ST_TIMEOUT]:
+            raise RuntimeError('halo exchange timed out waiting for a peer rank')
+        if st[L.DD_ST_BAD_INPUT]:
+            self.nl.check()
+            raise RuntimeError('neighbour list failure on a peer rank (degree overflow / singular cell)')
+        return st
 
     def halo_bytes_per_step(self):
         """Bytes this rank stores into peer memory per step (feature rows + forces), and the number of exchanges."""
@@ -477,6 +472,8 @@ class DomainDecomposition:
     dd = DomainDecomposition(model); out = dd(z, pos, cell)   (same full inputs on every rank)
     -> CustomOutputSet with energy [1], gradient_force [N,3] (complete on every rank), stress, virial.
     """
+
+    HEADROOM = (1.08, 64)          # eager path's edge capacity: factor and slack over the counted edges
 
     def __init__(self, model, group=None, grid=None, skin=1.0, transport='p2p', overlap=True, use_cuda_graph=True):
         """skin (A): the brick/ghost plan is kept while no atom has moved more than skin/2 since it was
@@ -503,12 +500,7 @@ class DomainDecomposition:
     def check(self):
         """Read the status of the last step (one small D2H copy, synchronises).  Returns the status words;
         raises on conditions that invalidate the result.  `__call__(..., sync=True)` does this itself."""
-        st = self._peer.out_status.cpu().tolist()
-        if st[L.DD_ST_TIMEOUT]:
-            raise RuntimeError('halo exchange timed out waiting for a peer rank')
-        if st[L.DD_ST_BAD_INPUT]:
-            self._peer.nl.check()
-            raise RuntimeError('neighbour list failure on a peer rank (degree overflow / singular cell)')
+        st = self._peer.status()
         if st[L.DD_ST_STALE]:
             raise RuntimeError('an atom moved more than skin/2 since the brick/ghost plan was made and the step ran with '
                                'sync=False: call with sync=True (replans automatically) or increase skin')
@@ -532,18 +524,12 @@ class DomainDecomposition:
             p.run(z, pos, cell3)
             if not sync:
                 break
-            st = p.out_status.cpu().tolist()            # the one host synchronisation of the step
-            if st[L.DD_ST_TIMEOUT]:
-                raise RuntimeError('halo exchange timed out waiting for a peer rank')
-            if st[L.DD_ST_BAD_INPUT]:
-                p.nl.check()
-                raise RuntimeError('neighbour list failure on a peer rank (degree overflow / singular cell)')
+            st = p.status()                             # the one host synchronisation of the step
             if st[L.DD_ST_STALE]:                        # same decision on every rank: the flags were OR-ed by nn_dd_finish
                 p.stale = True                           # re-cut the bricks for the new positions, keep arena and capacities
                 continue
             if st[L.DD_ST_OVERFLOW]:
-                need = p.nl.status.cpu().tolist()
-                p._size_neighbor_list(max(need[L.ST_EDGE_OVERFLOW], need[L.ST_N_EDGES]))
+                p._size_neighbor_list(edges_needed(p.nl.status.cpu().tolist()))
                 continue
             break
         else:
@@ -595,7 +581,6 @@ class DomainDecomposition:
         return self._call_eager(z, pos, cell, want_virial)
 
     def _call_eager(self, z, pos, cell, want_virial=True):
-        from newtonnet_b200.engine import NeighborList, _stream, get_engine
         from newtonnet_b200.models.output import CustomOutputSet
         model = self.model
         dev = pos.device
@@ -621,43 +606,27 @@ class DomainDecomposition:
         pos_l = pos.detach().to(torch.float32)[l2g].contiguous()
         cell_l = cell3.detach().to(torch.float32).contiguous()
         n_local, n_owned = int(l2g.shape[0]), plan.n_owned
-        s = _stream()
+        s = stream()
 
         # ---- neighbour list over owned + ghost atoms (ghost-ghost pairs dropped); capacities are kept
-        def build(cap):
-            # ghost rows of the list stay empty, so an owned-ghost pair has ONE directed edge: up to one pair per edge
-            nl = NeighborList(engine, pos_l, cell_l, batch_l, cap_edges=cap, cap_pairs=cap)
-            nl.struct.n_owned = n_owned
-            return nl
-
-        def run_nbr(nl, fill=True):
-            L.check(lib.nn_nbr_count(C.byref(nl.struct), pack.cutoff, s), 'nn_nbr_count')
-            if fill:
-                L.check(lib.nn_nbr_fill(C.byref(nl.struct), pack.cutoff, s), 'nn_nbr_fill')
-
         if self._nl is None:
-            probe = build(0)
-            run_nbr(probe, fill=False)
-            cap = int(probe.check()[L.ST_N_EDGES] * 1.08) + 64
-            self._nl = build(cap + cap % 2)
+            cap = edge_capacity(count_edges(engine, pos_l, cell_l, batch_l, pack.cutoff, n_owned).n_edges, *self.HEADROOM)
+            # ghost rows of the list stay empty, so an owned-ghost pair has ONE directed edge: up to one pair per edge
+            self._nl = NeighborList(engine, pos_l, cell_l, batch_l, cap, cap, n_owned)
         nl = self._nl
         nl.rebind(pos_l, cell_l, batch_l)
-        nl.n_edges = None
-        run_nbr(nl)
+        nl.rebuild(pack.cutoff)
         n_layers = pack.n_layers
 
         # ---- phased evaluation with halo exchanges
         f32 = dict(dtype=torch.float32, device=dev)
         energy = torch.zeros(1, **f32); forces_l = torch.zeros(max(n_owned, 1), 3, **f32)
         virial = torch.zeros(1, 3, 3, **f32); stress = torch.zeros(1, 3, 3, **f32)
-        nbytes = lib.nn_eval_workspace_bytes(n_local, 1, nl.cap_pairs, n_layers, 1)
-        ws = self._workspace(nbytes, dev)
-        a = L.EvalArgs()
-        a.nbr, a.w, a.z = C.pointer(nl.struct), C.pointer(pack.struct), z_l.data_ptr()
-        a.want_forces, a.want_virial, a.n_owned = 1, int(want_virial), n_owned
-        a.energy, a.forces = energy.data_ptr(), forces_l.data_ptr()
-        a.virial, a.stress = (virial.data_ptr(), stress.data_ptr()) if want_virial else (None, None)
-        a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
+        ws = self._workspace(lib.nn_eval_workspace_bytes(n_local, 1, nl.cap_pairs, n_layers, 1), dev)
+        outputs = {'energy': energy, 'forces': forces_l}
+        if want_virial:
+            outputs.update(virial=virial, stress=stress)
+        a = eval_args(nl, pack, z_l, outputs, ws, True, want_virial, n_owned)
 
         def phase(ph, l=0):
             L.check(lib.nn_eval_phase(C.byref(a), ph, l, s), f'nn_eval_phase({ph},{l})')

@@ -4,6 +4,7 @@ PyTorch is used for device memory and streams only; all arithmetic happens in
 libnewtonnet_b200.so (include/newtonnet_b200.h).
 """
 import ctypes as C
+import gc
 import os
 
 import torch
@@ -11,7 +12,8 @@ import torch
 from . import _lib as L
 
 
-def _stream():
+def stream():
+    """Raw handle of the current CUDA stream, as the library's entry points take it."""
     return torch.cuda.current_stream().cuda_stream
 
 
@@ -116,9 +118,10 @@ class WeightPack:
 class NeighborList:
     """Destination-sorted CSR + undirected pair list on the device (nn_nbr)."""
 
-    def __init__(self, engine, pos, cell, batch, cap_edges, cap_pairs=None):
+    def __init__(self, engine, pos, cell, batch, cap_edges, cap_pairs=None, n_owned=0):
         """cap_pairs: capacity of the pair table; default cap_edges / 2 (complete lists have P = E / 2 - lists with empty
-        ghost rows, domain decomposition, have up to P = E pairs and pass it explicitly)."""
+        ghost rows, domain decomposition, have up to P = E pairs and pass it explicitly).
+        n_owned > 0: atoms [n_owned, N) are ghosts, and pairs between two ghosts are left out."""
         N, B = pos.shape[0], cell.shape[0]
         dev = pos.device
         i32 = dict(dtype=torch.int32, device=dev)
@@ -140,6 +143,7 @@ class NeighborList:
         s = L.Nbr()
         s.n_atoms, s.n_systems = N, B
         s.cap_edges, s.cap_pairs, s.cap_cells = self.cap_edges, self.cap_pairs, 2 * N + B
+        s.n_owned = n_owned
         s.pos, s.cell, s.batch = pos.data_ptr(), cell.data_ptr(), batch.data_ptr()
         s.sys_ptr, s.row_ptr, s.col = self.sys_ptr.data_ptr(), self.row_ptr.data_ptr(), self.col.data_ptr()
         s.edge_pair, s.pair_ptr = self.edge_pair.data_ptr(), self.pair_ptr.data_ptr()
@@ -154,6 +158,13 @@ class NeighborList:
         """Point the list at new input tensors of the same shapes (next MD step)."""
         self.pos, self.cell, self.batch = pos, cell, batch
         self.struct.pos, self.struct.cell, self.struct.batch = pos.data_ptr(), cell.data_ptr(), batch.data_ptr()
+
+    def rebuild(self, cutoff):
+        """Count + fill on the current stream.  A list that outgrows its capacity is not filled: the status words say so."""
+        lib, s = L.load(), stream()
+        self.n_edges = None
+        L.check(lib.nn_nbr_count(C.byref(self.struct), cutoff, s), 'nn_nbr_count')
+        L.check(lib.nn_nbr_fill(C.byref(self.struct), cutoff, s), 'nn_nbr_fill')
 
     def check(self):
         """Read the status words (one small D2H copy, synchronises the stream)."""
@@ -183,15 +194,113 @@ class NeighborList:
         out = torch.empty(2, self.n_edges, dtype=torch.int64, device=self.pos.device)
         if self.n_edges:
             lib = L.load()
-            L.check(lib.nn_nbr_edge_index(C.byref(self.struct), out.data_ptr(), self.n_edges, _stream()), 'nn_nbr_edge_index')
+            L.check(lib.nn_nbr_edge_index(C.byref(self.struct), out.data_ptr(), self.n_edges, stream()), 'nn_nbr_edge_index')
         return out
+
+
+def count_edges(engine, pos, cell, batch, cutoff, n_owned=0):
+    """Count-only pass over a list of capacity 0.  Returns that list, checked: `n_edges` holds the directed edges the
+    inputs need, and `row_ptr` / `sys_ptr` the count per atom / per system."""
+    probe = NeighborList(engine, pos, cell, batch, cap_edges=0, n_owned=n_owned)
+    L.check(engine.lib.nn_nbr_count(C.byref(probe.struct), cutoff, stream()), 'nn_nbr_count')
+    probe.check()
+    return probe
+
+
+def edge_capacity(n_edges, factor, slack, bound=None):
+    """Edge capacity for `n_edges` edges: int(n_edges * factor) + slack, at most `bound`, made even and at least 2."""
+    c = int(n_edges * factor) + slack
+    if bound is not None:
+        c = min(c, bound)
+    return max(c + c % 2, 2)
+
+
+def edges_needed(status):
+    """Edges a list must hold after its status words reported an overflow."""
+    return max(status[L.ST_EDGE_OVERFLOW], status[L.ST_N_EDGES])
+
+
+def all_pairs_bound(cell, batch):
+    """Most directed edges a batch without a periodic cell can have: every ordered pair within each system.  None when a
+    cell is periodic (periodic images make pairs repeat)."""
+    if bool((cell != 0).any()):
+        return None
+    n = torch.bincount(batch, minlength=cell.shape[0])
+    return int((n * (n - 1)).sum())
+
+
+def eval_outputs(N, B, device, want_forces, want_virial, want_nodes, want_direct):
+    """The output tensors nn_eval writes for these requests (the virial needs the forces' reverse sweep)."""
+    f32 = dict(dtype=torch.float32, device=device)
+    out = {'energy': torch.empty(B, **f32)}
+    if want_forces or want_virial:
+        out['forces'] = torch.empty(N, 3, **f32)
+    if want_virial:
+        out['virial'] = torch.empty(B, 3, 3, **f32)
+        out['stress'] = torch.empty(B, 3, 3, **f32)
+    if want_nodes:
+        out['atom_node'] = torch.empty(N, L.NN_F, **f32)
+        out['force_node'] = torch.empty(N, 3, L.NN_F, **f32)
+    if want_direct:
+        out['direct_force'] = torch.empty(N, 3, **f32)
+    return out
+
+
+def eval_args(nl, weights, z, out, ws, want_forces, want_virial, n_owned=0):
+    """nn_eval's arguments: outputs are the tensors of `out` (a missing key passes NULL), `ws` is the workspace."""
+    a = L.EvalArgs()
+    a.nbr, a.w, a.z = C.pointer(nl.struct), C.pointer(weights.struct), z.data_ptr()
+    a.want_forces, a.want_virial, a.n_owned = int(want_forces or want_virial), int(want_virial), n_owned
+    a.energy = out['energy'].data_ptr()
+    for k in ('forces', 'virial', 'stress', 'atom_node', 'force_node', 'direct_force'):
+        setattr(a, k, L.ptr(out.get(k)))
+    a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
+    return a
+
+
+class _gc_paused:
+    """Python's cyclic collector off while a graph is captured.  Collected cycles may own CUDA graphs or events; destroying
+    one while a capture is running is not a stream operation and invalidates the capture.  torch.cuda.graph no longer
+    collects before it captures."""
+
+    def __enter__(self):
+        self.was = gc.isenabled()
+        gc.disable()
+
+    def __exit__(self, *exc):
+        if self.was:
+            gc.enable()
+        return False
+
+
+def capture(fn, device, pool=None):
+    """Synchronise the device, then capture fn() as a CUDA graph with the cyclic collector paused.  Returns (graph, what
+    fn returned, launches of this library the graph holds)."""
+    lib = L.load()
+    torch.cuda.synchronize(device)
+    graph = torch.cuda.CUDAGraph()
+    before = lib.nn_launch_count(0)
+    with _gc_paused(), torch.cuda.graph(graph, pool=pool):
+        result = fn()
+    return graph, result, int(lib.nn_launch_count(0) - before)
+
+
+def warm_up(fn, device, times):
+    """Run fn() `times` times on a side stream that then joins the current one: the warm-up torch asks for before a
+    capture, so that lazy initialisation does not happen inside it."""
+    side = torch.cuda.Stream(device=device)
+    side.wait_stream(torch.cuda.current_stream(device))
+    with torch.cuda.stream(side):
+        for _ in range(times):
+            fn()
+    torch.cuda.current_stream(device).wait_stream(side)
 
 
 class Engine:
     """Per-device driver.  Keeps capacities and workspaces between calls so a steady-state evaluation
     allocates nothing and synchronises once (the status read that accompanies the results)."""
 
-    HEADROOM = 1.08
+    HEADROOM = (1.08, 64)          # edge capacity: factor and slack over the counted edges
 
     def __init__(self, device):
         self.device = torch.device(device)
@@ -200,7 +309,6 @@ class Engine:
         self.lib = L.load()
         self._nl = None
         self._ws = None
-        self.launches = 0
         self.use_cuda_graphs = os.environ.get('NN_CUDA_GRAPHS', '1') != '0'
         self._graphs = {}
         self._last_key = None
@@ -215,31 +323,18 @@ class Engine:
         N, B = pos.shape[0], cell.shape[0]
         nl = self._nl
         reuse = nl is not None and nl.n_atoms == N and nl.n_systems == B and nl.pos.device == pos.device
-        s = _stream()
         if reuse:
             nl.rebind(pos, cell, batch)
-            nl.n_edges = None
             nl.generation += 1
-            L.check(self.lib.nn_nbr_count(C.byref(nl.struct), cutoff, s), 'nn_nbr_count')
-            L.check(self.lib.nn_nbr_fill(C.byref(nl.struct), cutoff, s), 'nn_nbr_fill')
-            return nl   # overflow (if any) is detected by the caller's status check -> `grow`
-        probe = NeighborList(self, pos, cell, batch, cap_edges=0)
-        L.check(self.lib.nn_nbr_count(C.byref(probe.struct), cutoff, s), 'nn_nbr_count')
-        st = probe.check()
-        return self._build_with_capacity(pos, cell, batch, cutoff, st[L.ST_N_EDGES])
+            nl.rebuild(cutoff)
+            return nl   # overflow (if any) is detected by the caller's status check
+        return self._build_with_capacity(pos, cell, batch, cutoff, count_edges(self, pos, cell, batch, cutoff).n_edges)
 
     def _build_with_capacity(self, pos, cell, batch, cutoff, n_edges):
-        cap = int(n_edges * self.HEADROOM) + 64
-        cap += cap % 2
-        nl = NeighborList(self, pos, cell, batch, cap_edges=cap)
-        s = _stream()
-        L.check(self.lib.nn_nbr_count(C.byref(nl.struct), cutoff, s), 'nn_nbr_count')
-        L.check(self.lib.nn_nbr_fill(C.byref(nl.struct), cutoff, s), 'nn_nbr_fill')
+        nl = NeighborList(self, pos, cell, batch, cap_edges=edge_capacity(n_edges, *self.HEADROOM))
+        nl.rebuild(cutoff)
         self._nl = nl
         return nl
-
-    def grow(self, nl, cutoff, needed):
-        return self._build_with_capacity(nl.pos, nl.cell, nl.batch, cutoff, needed)
 
     def checked_neighbor_list(self, pos, cell, batch, cutoff):
         """neighbor_list + status read; a cached list whose capacity the new positions outgrow is rebuilt larger
@@ -247,7 +342,7 @@ class Engine:
         nl = self.neighbor_list(pos, cell, batch, cutoff)
         st = nl.check()
         if st[L.ST_EDGE_OVERFLOW]:
-            nl = self.grow(nl, cutoff, max(st[L.ST_EDGE_OVERFLOW], st[L.ST_N_EDGES]))
+            nl = self._build_with_capacity(nl.pos, nl.cell, nl.batch, cutoff, edges_needed(st))
             st = nl.check()
             if st[L.ST_EDGE_OVERFLOW]:
                 raise RuntimeError('neighbour list capacity overflow after regrow')
@@ -262,37 +357,11 @@ class Engine:
     def evaluate(self, nl, weights, z, want_forces=True, want_virial=False, want_nodes=False, want_direct=False):
         _require_cuda(z, 'z')
         z = z.to(torch.int64).contiguous()
-        N, B = nl.n_atoms, nl.n_systems
-        dev = nl.pos.device
-        f32 = dict(dtype=torch.float32, device=dev)
-        out = {'energy': torch.empty(B, **f32)}
-        bwd = want_forces or want_virial
-        if bwd:
-            out['forces'] = torch.empty(N, 3, **f32)
-        if want_virial:
-            out['virial'] = torch.empty(B, 3, 3, **f32)
-            out['stress'] = torch.empty(B, 3, 3, **f32)
-        if want_nodes:
-            out['atom_node'] = torch.empty(N, L.NN_F, **f32)
-            out['force_node'] = torch.empty(N, 3, L.NN_F, **f32)
-        if want_direct:
-            out['direct_force'] = torch.empty(N, 3, **f32)
-        nbytes = self.lib.nn_eval_workspace_bytes(N, B, nl.cap_pairs, weights.n_layers, int(bwd))
-        ws = self._workspace(nbytes)
-        a = L.EvalArgs()
-        a.nbr = C.pointer(nl.struct)
-        a.w = C.pointer(weights.struct)
-        a.z = z.data_ptr()
-        a.want_forces, a.want_virial = int(bwd), int(want_virial)
-        a.energy = out['energy'].data_ptr()
-        a.forces = L.ptr(out.get('forces'))
-        a.virial = L.ptr(out.get('virial'))
-        a.stress = L.ptr(out.get('stress'))
-        a.atom_node = L.ptr(out.get('atom_node'))
-        a.force_node = L.ptr(out.get('force_node'))
-        a.direct_force = L.ptr(out.get('direct_force'))
-        a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
-        L.check(self.lib.nn_eval(C.byref(a), _stream()), 'nn_eval')
+        out = eval_outputs(nl.n_atoms, nl.n_systems, nl.pos.device, want_forces, want_virial, want_nodes, want_direct)
+        ws = self._workspace(self.lib.nn_eval_workspace_bytes(nl.n_atoms, nl.n_systems, nl.cap_pairs, weights.n_layers,
+                                                              int(want_forces or want_virial)))
+        a = eval_args(nl, weights, z, out, ws, want_forces, want_virial)
+        L.check(self.lib.nn_eval(C.byref(a), stream()), 'nn_eval')
         out['_z'] = z   # keep alive until the stream has consumed it
         return out
 
@@ -324,7 +393,7 @@ class Engine:
         out = self.evaluate(nl, weights, z, want_forces, want_virial, want_nodes, want_direct)
         st = nl.check()
         if st[L.ST_EDGE_OVERFLOW]:
-            nl = self.grow(nl, weights.cutoff, max(st[L.ST_EDGE_OVERFLOW], st[L.ST_N_EDGES]))
+            nl = self._build_with_capacity(nl.pos, nl.cell, nl.batch, weights.cutoff, edges_needed(st))
             out = self.evaluate(nl, weights, z, want_forces, want_virial, want_nodes, want_direct)
             st = nl.check()
             if st[L.ST_EDGE_OVERFLOW]:
@@ -347,40 +416,15 @@ class GraphedStep:
         self._copy_in(z, pos, cell, batch)
         self.nl = NeighborList(engine, self.pos, self.cell, self.batch, cap_edges=cap_edges)
         N, B = self.nl.n_atoms, self.nl.n_systems
-        f32 = dict(dtype=torch.float32, device=dev)
-        bwd = want_forces or want_virial
-        self.out = {'energy': torch.empty(B, **f32)}
-        if bwd:
-            self.out['forces'] = torch.empty(N, 3, **f32)
-        if want_virial:
-            self.out['virial'] = torch.empty(B, 3, 3, **f32)
-            self.out['stress'] = torch.empty(B, 3, 3, **f32)
-        if want_nodes:
-            self.out['atom_node'] = torch.empty(N, L.NN_F, **f32)
-            self.out['force_node'] = torch.empty(N, 3, L.NN_F, **f32)
-        if want_direct:
-            self.out['direct_force'] = torch.empty(N, 3, **f32)
-        nbytes = engine.lib.nn_eval_workspace_bytes(N, B, self.nl.cap_pairs, weights.n_layers, int(bwd))
+        self.out = eval_outputs(N, B, dev, want_forces, want_virial, want_nodes, want_direct)
+        nbytes = engine.lib.nn_eval_workspace_bytes(N, B, self.nl.cap_pairs, weights.n_layers, int(want_forces or want_virial))
         self.ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=dev)
-        a = L.EvalArgs()
-        a.nbr, a.w, a.z = C.pointer(self.nl.struct), C.pointer(weights.struct), self.z.data_ptr()
-        a.want_forces, a.want_virial = int(bwd), int(want_virial)
-        a.energy = self.out['energy'].data_ptr()
-        a.forces, a.virial, a.stress = L.ptr(self.out.get('forces')), L.ptr(self.out.get('virial')), L.ptr(self.out.get('stress'))
-        a.atom_node, a.force_node = L.ptr(self.out.get('atom_node')), L.ptr(self.out.get('force_node'))
-        a.direct_force = L.ptr(self.out.get('direct_force'))
-        a.workspace, a.workspace_bytes = self.ws.data_ptr(), self.ws.numel()
-        self.args = a
-        torch.cuda.synchronize(dev)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            self._launch()
+        self.args = eval_args(self.nl, weights, self.z, self.out, self.ws, want_forces, want_virial)
+        self.graph, _, _ = capture(self._launch, dev)
 
     def _launch(self):
-        lib, s = self.engine.lib, _stream()
-        L.check(lib.nn_nbr_count(C.byref(self.nl.struct), self.weights.cutoff, s), 'nn_nbr_count')
-        L.check(lib.nn_nbr_fill(C.byref(self.nl.struct), self.weights.cutoff, s), 'nn_nbr_fill')
-        L.check(lib.nn_eval(C.byref(self.args), s), 'nn_eval')
+        self.nl.rebuild(self.weights.cutoff)
+        L.check(self.engine.lib.nn_eval(C.byref(self.args), stream()), 'nn_eval')
 
     def _copy_in(self, z, pos, cell, batch):
         self.z.copy_(z, non_blocking=True)

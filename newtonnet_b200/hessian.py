@@ -22,14 +22,13 @@ budget, parameter addresses) and reused when the same molecule comes back at new
 GraphedTrainingStep; a pass whose list outgrows it leaves a flag that is read after the group's replays, and the group is
 then recaptured with more room and run again.  NN_HESSIAN_GRAPH=0 runs the same passes eagerly.
 """
-import ctypes as C
-import gc
 import os
 
 import numpy as np
 import torch
 
 from . import _lib as L
+from .engine import NeighborList, all_pairs_bound, capture, count_edges, edge_capacity, get_engine, stream, warm_up
 
 # Device memory one replicated atom costs on the differentiable path (forward + create_graph backward + second backward):
 # peak allocated bytes of a call over the atoms of its largest pass, MEASURED with tools/bench_hessian.py on a B200
@@ -111,29 +110,12 @@ def default_budget(device):
 
 
 # ----------------------------------------------------------------------------- device side
-def _stream():
-    return torch.cuda.current_stream().cuda_stream
-
-
-class _gc_paused:
-    """Python's cyclic collector off while a graph is captured.  Collected cycles may own CUDA graphs or events (this
-    module's are freed by reference count, a caller's objects need not be); destroying one while a capture is running
-    is not a stream operation and invalidates the capture.  torch.cuda.graph no longer collects before it captures."""
-
-    def __enter__(self):
-        self.was = gc.isenabled()
-        gc.disable()
-
-    def __exit__(self, *exc):
-        if self.was:
-            gc.enable()
-        return False
-
-
 class _GroupRunner:
     """The passes of one group on static buffers; one CUDA graph replayed once per pass (or the same pass run eagerly).
     It holds no reference to its _Blocks (which is passed in): an evicted _Blocks then frees its graphs at once, by
     reference count, instead of whenever the cyclic collector runs - possibly in the middle of a later capture."""
+
+    HEADROOM = (1.05, 256)         # tight edge capacity, as in GraphedTrainingStep: factor and slack over the counted edges
 
     def __init__(self, b, group, max_edges):
         dev = b.device
@@ -145,46 +127,35 @@ class _GroupRunner:
         self.cell_rep = torch.empty(k, 3, 3, dtype=torch.float32, device=dev)
         self.batch_rep = torch.empty(k * n, dtype=torch.int64, device=dev)
         self.seed = torch.empty(k * n, 3, dtype=torch.float32, device=dev)
-        self.periodic = b.periodic
+        self.bound = all_pairs_bound(b.cell, torch.arange(k).repeat_interleave(n))     # k copies of an n-atom frame
         self.graph = None
         self.recaptures = 0
-        self._build(b, self._headroom(k * max_edges))
+        self._build(b, self._capacity(k * max_edges))
 
-    def _headroom(self, n_edges):
-        cap = int(n_edges * 1.05) + 256
-        if not self.periodic:                          # all ordered pairs within each copy bound the list
-            cap = min(cap, self.group.k * self.group.n * (self.group.n - 1))
-        return max(cap + cap % 2, 2)
+    def _capacity(self, n_edges):
+        return edge_capacity(n_edges, *self.HEADROOM, self.bound)
 
     def _build(self, b, cap_edges):
-        from newtonnet_b200.engine import NeighborList
         self.graph = None                              # the previous capture's graph goes first
         self.nl = NeighborList(b.engine, self.pos_rep, self.cell_rep, self.batch_rep, cap_edges=cap_edges)
         if not b.graphed:
             return
-        dev = b.device
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):                  # warm-up on a side stream, as graph capture requires
+
+        def first_pass():
             b.ctr.zero_()
             self._pass(b)
-        torch.cuda.current_stream(dev).wait_stream(side)
-        torch.cuda.synchronize(dev)
-        graph = torch.cuda.CUDAGraph()
-        with _gc_paused(), torch.cuda.graph(graph, pool=b.pool):
-            self._pass(b)
-        self.graph = graph
+        warm_up(first_pass, b.device, 1)
+        self.graph, _, _ = capture(lambda: self._pass(b), b.device, pool=b.pool)
         stats['captures'] += 1
 
     def _pass(self, b):
         from newtonnet_b200.train import _skip_weight_grads, differentiable_forward
-        g, lib, s = self.group, b.lib, _stream()
+        g, lib, s = self.group, b.lib, stream()
         L.check(lib.nn_hessian_expand(self.plan.data_ptr(), b.ctr.data_ptr(), g.k, g.n, b.z.data_ptr(), b.pos.data_ptr(),
                                       b.cell.data_ptr(), b.frame_ptr.data_ptr(), self.z_rep.data_ptr(), self.pos_rep.data_ptr(),
                                       self.cell_rep.data_ptr(), self.batch_rep.data_ptr(), self.seed.data_ptr(), s),
                 'nn_hessian_expand')
-        L.check(lib.nn_nbr_count(C.byref(self.nl.struct), b.model.cutoff, s), 'nn_nbr_count')
-        L.check(lib.nn_nbr_fill(C.byref(self.nl.struct), b.model.cutoff, s), 'nn_nbr_fill')
+        self.nl.rebuild(b.model.cutoff)
         pos = self.pos_rep.detach().requires_grad_(True)
         out = differentiable_forward(b.model, self.z_rep, pos, self.cell_rep, self.batch_rep, static_nl=self.nl,
                                      properties=('energy',))
@@ -211,7 +182,7 @@ class _GroupRunner:
                 return
             if attempt == 3:
                 break
-            self._build(b, max(self._headroom(need), self.nl.cap_edges + 2))
+            self._build(b, max(self._capacity(need), self.nl.cap_edges + 2))
             self.recaptures += 1
         raise RuntimeError(f'Hessian pass: edge capacity {self.nl.cap_edges} still overflowed after regrowing')
 
@@ -220,7 +191,6 @@ class _Blocks:
     """Static inputs / output of one Hessian shape and the runners of its groups."""
 
     def __init__(self, model, z, pos, cell, batch, frame_sizes, atoms, budget, graphed):
-        from newtonnet_b200.engine import NeighborList, get_engine
         dev = pos.device
         self.model, self.device, self.graphed = model, dev, graphed
         self.engine = get_engine(dev)
@@ -238,11 +208,8 @@ class _Blocks:
         self.sticky = torch.zeros(1, **i32)
         self.pool = torch.cuda.graph_pool_handle() if graphed else None     # one pool for the groups' graphs
         self.copy_in(z, pos, cell)
-        self.periodic = bool((self.cell != 0).any())
         # edges per frame from a counting pass over the input batch size the first capture
-        probe = NeighborList(self.engine, self.pos, self.cell, batch.to(torch.int64).contiguous(), cap_edges=0)
-        L.check(self.lib.nn_nbr_count(C.byref(probe.struct), model.cutoff, _stream()), 'nn_nbr_count')
-        probe.check()
+        probe = count_edges(self.engine, self.pos, self.cell, batch.to(torch.int64).contiguous(), model.cutoff)
         per_frame = (probe.row_ptr[probe.sys_ptr[1:].long()] - probe.row_ptr[probe.sys_ptr[:-1].long()]).cpu().numpy()
         self.runners = []
         for g in self.groups:

@@ -78,7 +78,7 @@ class EdgeEmbedding(nn.Module):
     def forward(self, pos, cell=None, batch=None):
         """-> (dist_edge [E,n_basis], dir_edge [E,3], edge_index [2,E]) as representations.py:20-43."""
         from newtonnet_b200 import _lib as L
-        from newtonnet_b200.engine import _stream
+        from newtonnet_b200.engine import stream
         edge_index, disp = self.radius_graph(pos, cell, batch)
         E = disp.shape[0]
         dev = pos.device
@@ -89,6 +89,6 @@ class EdgeEmbedding(nn.Module):
         freq = self.embedding.frequencies.detach().to(device=dev, dtype=torch.float32).contiguous()
         if E:
             L.check(L.load().nn_edge_geom_fwd(d32.data_ptr(), freq.data_ptr(), float(self.norm.r), None, E,
-                                             rbf.data_ptr(), None, unit.data_ptr(), dist.data_ptr(), _stream()),
+                                             rbf.data_ptr(), None, unit.data_ptr(), dist.data_ptr(), stream()),
                     'nn_edge_geom_fwd')
         return rbf.to(pos.dtype), unit.to(pos.dtype), edge_index

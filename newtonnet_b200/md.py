@@ -19,7 +19,7 @@ import numpy as np
 import torch
 
 from newtonnet_b200 import _lib as L
-from newtonnet_b200.engine import NeighborList, get_engine
+from newtonnet_b200.engine import NeighborList, capture, count_edges, edge_capacity, edges_needed, eval_args, get_engine, stream
 
 __all__ = ['DeviceMD', 'FS', 'KB', 'ATOMIC_MASSES']
 
@@ -31,10 +31,6 @@ ATOMIC_MASSES = np.array([0.0, 1.008, 4.002602, 6.94, 9.0121831, 10.81, 12.011, 
                           69.723, 72.630, 74.921595, 78.971, 79.904, 83.798])
 
 
-def _stream():
-    return torch.cuda.current_stream().cuda_stream
-
-
 class DeviceMD:
     """NVE / Langevin MD of one system or a batch of independent systems, state resident on the GPU.
 
@@ -43,7 +39,7 @@ class DeviceMD:
     temperature_K + friction (1 / ASE time) switch the Ornstein-Uhlenbeck step on; velocities [N,3] or None
     (Maxwell-Boltzmann at temperature_K when given, else zero)."""
 
-    HEADROOM = 1.15
+    HEADROOM = (1.15, 64)          # edge capacity: factor and slack over the counted edges
 
     def __init__(self, model, z, pos, cell=None, batch=None, masses=None, timestep=0.5 * FS, temperature_K=None,
                  friction=None, velocities=None, seed=0, log_capacity=1024, check_interval=64):
@@ -94,10 +90,7 @@ class DeviceMD:
         self.log = torch.zeros(self.log_capacity, B, 2, dtype=torch.float64, device=dev)
         self.graph_launches = 0
         self._wrap()
-        probe = NeighborList(self.engine, self.pos_model, self.cell, self.batch, cap_edges=0)
-        L.check(self.lib.nn_nbr_count(C.byref(probe.struct), self.weights.cutoff, _stream()), 'nn_nbr_count')
-        st = probe.check()
-        self._build(st[L.ST_N_EDGES])
+        self._build(count_edges(self.engine, self.pos_model, self.cell, self.batch, self.weights.cutoff).n_edges)
 
     # ------------------------------------------------------------------ construction helpers
     @classmethod
@@ -122,48 +115,37 @@ class DeviceMD:
         L.check(self.lib.nn_md_advance(self.n_atoms, self.x.data_ptr(), self.v.data_ptr(), self.force.data_ptr(),
                                        self.inv_mass.data_ptr(), self.cell.data_ptr(), self.batch.data_ptr(),
                                        self.pos_model.data_ptr(), dt, ou_c, self.kT, self.seed, self.step_ctr.data_ptr(),
-                                       _stream()), 'nn_md_advance')
+                                       stream()), 'nn_md_advance')
 
     def _wrap(self):
         self._advance(0.0, 1.0)          # zero time step: only writes the wrapped fp32 copy
 
     def _forces(self):
-        s = _stream()
-        L.check(self.lib.nn_nbr_count(C.byref(self.nl.struct), self.weights.cutoff, s), 'nn_nbr_count')
-        L.check(self.lib.nn_nbr_fill(C.byref(self.nl.struct), self.weights.cutoff, s), 'nn_nbr_fill')
-        L.check(self.lib.nn_eval(C.byref(self.args), s), 'nn_eval')
+        self.nl.rebuild(self.weights.cutoff)
+        L.check(self.lib.nn_eval(C.byref(self.args), stream()), 'nn_eval')
 
     def _finish(self):
         L.check(self.lib.nn_md_finish(self.n_systems, self.nl.sys_ptr.data_ptr(), self.v.data_ptr(), self.force.data_ptr(),
                                       self.inv_mass.data_ptr(), self.dt, self.energy.data_ptr(), self.log.data_ptr(),
                                       self.log_capacity, self.step_ctr.data_ptr(), self.nl.status.data_ptr(),
-                                      self.sticky.data_ptr(), self.ticket.data_ptr(), _stream()), 'nn_md_finish')
+                                      self.sticky.data_ptr(), self.ticket.data_ptr(), stream()), 'nn_md_finish')
+
+    def _step(self):
+        self._advance(self.dt, self.ou_c)
+        self._forces()
+        self._finish()
 
     def _build(self, n_edges):
         """(Re)allocate the neighbour list for `n_edges`, evaluate forces at the current positions and capture the step."""
-        cap = int(n_edges * self.HEADROOM) + 64
-        cap += cap % 2
-        self.nl = NeighborList(self.engine, self.pos_model, self.cell, self.batch, cap_edges=cap)
+        self.nl = NeighborList(self.engine, self.pos_model, self.cell, self.batch, cap_edges=edge_capacity(n_edges, *self.HEADROOM))
         nbytes = self.lib.nn_eval_workspace_bytes(self.n_atoms, self.n_systems, self.nl.cap_pairs, self.weights.n_layers, 1)
         self.ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-        a = L.EvalArgs()
-        a.nbr, a.w, a.z = C.pointer(self.nl.struct), C.pointer(self.weights.struct), self.z.data_ptr()
-        a.want_forces, a.want_virial = 1, 0
-        a.energy, a.forces = self.energy.data_ptr(), self.force.data_ptr()
-        a.workspace, a.workspace_bytes = self.ws.data_ptr(), self.ws.numel()
-        self.args = a
+        self.args = eval_args(self.nl, self.weights, self.z, {'energy': self.energy, 'forces': self.force}, self.ws, True, False)
         self._forces()
         st = self.nl.check()
         if st[L.ST_EDGE_OVERFLOW]:
-            return self._build(max(st[L.ST_EDGE_OVERFLOW], st[L.ST_N_EDGES]))
-        torch.cuda.synchronize(self.device)
-        self.graph = torch.cuda.CUDAGraph()
-        before = self.lib.nn_launch_count(0)
-        with torch.cuda.graph(self.graph):
-            self._advance(self.dt, self.ou_c)
-            self._forces()
-            self._finish()
-        self.kernels_per_step = int(self.lib.nn_launch_count(0) - before)     # kernels one graph replay launches
+            return self._build(edges_needed(st))
+        self.graph, _, self.kernels_per_step = capture(self._step, self.device)     # kernels one graph replay launches
 
     # ------------------------------------------------------------------ run
     def run(self, steps, trajectory_interval=None):

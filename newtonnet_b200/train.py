@@ -24,10 +24,7 @@ import torch.distributed as dist
 import torch.nn.functional as Fn
 
 from . import _lib as L
-
-
-def _stream():
-    return torch.cuda.current_stream().cuda_stream
+from .engine import NeighborList, all_pairs_bound, capture, count_edges, edge_capacity, get_engine, stream, warm_up
 
 
 # ----------------------------------------------------------------------------- raw kernel calls
@@ -62,7 +59,7 @@ def prepare_weight_images(model):
             k = 2 * i + t
             src[k], img[k], tr[k] = p.data_ptr(), imgs[k].data_ptr(), t
             _image_cache[_image_key(p.t() if t else p)] = imgs[k]
-    L.check(lib.nn_gemm128_prepare_b_batch(src, tr, img, n, _stream()), 'nn_gemm128_prepare_b_batch')
+    L.check(lib.nn_gemm128_prepare_b_batch(src, tr, img, n, stream()), 'nn_gemm128_prepare_b_batch')
 
 
 def _operand_image(B):
@@ -74,7 +71,7 @@ def _operand_image(B):
             return img
     Bc = _c(B)
     img = torch.empty(L.NN_B_IMAGE_FLOATS, dtype=torch.float32, device=Bc.device)
-    L.check(L.load().nn_gemm128_prepare_b(Bc.data_ptr(), img.data_ptr(), _stream()), 'nn_gemm128_prepare_b')
+    L.check(L.load().nn_gemm128_prepare_b(Bc.data_ptr(), img.data_ptr(), stream()), 'nn_gemm128_prepare_b')
     if key is not None:
         _image_cache[key] = img
     return img
@@ -91,7 +88,7 @@ def _gemm_raw(X, B):
     # the row-major matrix itself is read by the SIMT back-end only; the tensor-core back-ends take the image
     Bm = _c(B) if lib.nn_get_gemm_backend() == 0 else B
     a.X, a.B, a.B_img, a.Y, a.m = X.data_ptr(), Bm.data_ptr(), img.data_ptr(), Y.data_ptr(), M
-    L.check(lib.nn_gemm128(C.byref(a), _stream()), 'nn_gemm128')
+    L.check(lib.nn_gemm128(C.byref(a), stream()), 'nn_gemm128')
     return Y
 
 
@@ -100,7 +97,7 @@ def _gemm_tn_raw(X, Y):
     M = X.shape[0]
     out = torch.empty(128, 128, dtype=torch.float32, device=X.device)
     ws = torch.empty(max(lib.nn_gemm128_tn_workspace_bytes(M), 4), dtype=torch.uint8, device=X.device)
-    L.check(lib.nn_gemm128_tn(X.data_ptr(), Y.data_ptr(), M, out.data_ptr(), ws.data_ptr(), _stream()), 'nn_gemm128_tn')
+    L.check(lib.nn_gemm128_tn(X.data_ptr(), Y.data_ptr(), M, out.data_ptr(), ws.data_ptr(), stream()), 'nn_gemm128_tn')
     return out
 
 
@@ -312,7 +309,7 @@ class Gather(torch.autograd.Function):
         n, width = seg.idx.shape[0], rows.shape[1]
         out = torch.empty(n, width, dtype=torch.float32, device=rows.device)
         if n:
-            L.check(L.load().nn_halo_pack(rows.data_ptr(), seg.idx.data_ptr(), n, width, out.data_ptr(), _stream()),
+            L.check(L.load().nn_halo_pack(rows.data_ptr(), seg.idx.data_ptr(), n, width, out.data_ptr(), stream()),
                     'nn_halo_pack')
         return out
 
@@ -333,7 +330,7 @@ class SegmentSum(torch.autograd.Function):
         out = (torch.empty if src.shape[0] else torch.zeros)(seg.n_rows, width, dtype=torch.float32, device=src.device)
         if src.shape[0]:
             L.check(L.load().nn_segment_sum(src.data_ptr(), L.ptr(seg.perm), seg.row_ptr.data_ptr(), seg.n_rows, width,
-                                            out.data_ptr(), _stream()), 'nn_segment_sum')
+                                            out.data_ptr(), stream()), 'nn_segment_sum')
         return out
 
     @staticmethod
@@ -349,7 +346,7 @@ def _rows(mode, p, q3, u, out_shape):
     out = torch.empty(out_shape, dtype=torch.float32, device=ref.device)
     n = out_shape[0]
     if n:
-        L.check(L.load().nn_ew_rows(mode, L.ptr(p), L.ptr(q3), L.ptr(u), out.data_ptr(), n, _stream()), 'nn_ew_rows')
+        L.check(L.load().nn_ew_rows(mode, L.ptr(p), L.ptr(q3), L.ptr(u), out.data_ptr(), n, stream()), 'nn_ew_rows')
     return out
 
 
@@ -362,7 +359,7 @@ class Mul3(torch.autograd.Function):
         a, b, c = _c(a), _c(b), _c(c)
         out = torch.empty_like(a)
         if a.numel():
-            L.check(L.load().nn_ew_mul3(a.data_ptr(), b.data_ptr(), c.data_ptr(), out.data_ptr(), a.numel(), _stream()), 'nn_ew_mul3')
+            L.check(L.load().nn_ew_mul3(a.data_ptr(), b.data_ptr(), c.data_ptr(), out.data_ptr(), a.numel(), stream()), 'nn_ew_mul3')
         return out
 
     @staticmethod
@@ -454,7 +451,7 @@ def _gmul_raw(a, b, r1, seg1, r2, seg2):
         r1 = _c(r1)
         r2 = None if r2 is None else _c(r2)
         L.check(L.load().nn_ew_gmul(a.data_ptr(), L.ptr(b), r1.data_ptr(), seg1.idx.data_ptr(), L.ptr(r2),
-                                    None if r2 is None else seg2.idx.data_ptr(), out.data_ptr(), n, _stream()), 'nn_ew_gmul')
+                                    None if r2 is None else seg2.idx.data_ptr(), out.data_ptr(), n, stream()), 'nn_ew_gmul')
     return out
 
 
@@ -504,7 +501,7 @@ def _seg_prod_raw(x, u, rows3, seg_in, seg_out):
     if x.shape[0]:
         L.check(L.load().nn_seg_prod(x.data_ptr(), None if u is None else _c(u).data_ptr(), None if rows3 is None else _c(rows3).data_ptr(),
                                      None if seg_in is None else seg_in.idx.data_ptr(), L.ptr(seg_out.perm), seg_out.row_ptr.data_ptr(),
-                                     seg_out.n_rows, out.data_ptr(), _stream()), 'nn_seg_prod')
+                                     seg_out.n_rows, out.data_ptr(), stream()), 'nn_seg_prod')
     return out
 
 
@@ -513,7 +510,7 @@ def _g3_raw(mode, rows3, seg, p, rowsb, segb, out_shape):
     if out_shape[0]:
         L.check(L.load().nn_ew_g3(mode, _c(rows3).data_ptr(), seg.idx.data_ptr(), None if p is None else _c(p).data_ptr(),
                                   None if rowsb is None else _c(rowsb).data_ptr(), None if segb is None else segb.idx.data_ptr(),
-                                  out.data_ptr(), out_shape[0], _stream()), 'nn_ew_g3')
+                                  out.data_ptr(), out_shape[0], stream()), 'nn_ew_g3')
     return out
 
 
@@ -608,7 +605,7 @@ def _rbf_raw(op, k, a, x, freq):
     n = x.shape[0]
     out = torch.empty((n, L.NN_NB) if op == 0 else (n, 1), dtype=torch.float32, device=x.device)
     if n:
-        L.check(L.load().nn_ew_rbf(op, k, L.ptr(None if a is None else _c(a)), x.data_ptr(), freq.data_ptr(), out.data_ptr(), n, _stream()),
+        L.check(L.load().nn_ew_rbf(op, k, L.ptr(None if a is None else _c(a)), x.data_ptr(), freq.data_ptr(), out.data_ptr(), n, stream()),
                 'nn_ew_rbf')
     return out
 
@@ -652,7 +649,7 @@ def _silu_raw(mode, x, a=None, b=None):
     out = torch.empty_like(x)
     if x.numel():
         L.check(L.load().nn_ew_silu(mode, x.data_ptr(), L.ptr(None if a is None else _c(a)), L.ptr(None if b is None else _c(b)),
-                                    out.data_ptr(), x.numel(), _stream()), 'nn_ew_silu')
+                                    out.data_ptr(), x.numel(), stream()), 'nn_ew_silu')
     return out
 
 
@@ -718,7 +715,7 @@ def _edges(nl, pos, N, static):
     else:
         E = nl.cap_edges
         ei = torch.zeros(2, E, dtype=torch.int64, device=pos.device)
-        L.check(L.load().nn_nbr_edge_index(C.byref(nl.struct), ei.data_ptr(), E, _stream()), 'nn_nbr_edge_index')
+        L.check(L.load().nn_nbr_edge_index(C.byref(nl.struct), ei.data_ptr(), E, stream()), 'nn_nbr_edge_index')
         # a list that outgrew its capacity was not (re)written: expose NO valid rows (the step then computes exact zeros from
         # padding instead of indexing with stale / uninitialised entries) - the caller reads the overflow flag afterwards
         n_valid = torch.where(nl.status[L.ST_EDGE_OVERFLOW] != 0, torch.zeros_like(nl.status[L.ST_N_EDGES]), nl.status[L.ST_N_EDGES])
@@ -768,7 +765,6 @@ def differentiable_forward(model, z, pos, cell, batch, static_nl=None, propertie
     static_nl: a NeighborList of fixed capacity already rebuilt for `pos` on the current stream -> the whole forward
     has static shapes and no host synchronisation (GraphedTrainingStep).
     properties: the outputs to form (default: model.output_properties; heads are looked up in the model's own list)."""
-    from newtonnet_b200.engine import get_engine
     from newtonnet_b200.models.output import CustomOutputSet
     own = list(model.output_properties)
     props = own if properties is None else list(properties)
@@ -796,7 +792,7 @@ def differentiable_forward(model, z, pos, cell, batch, static_nl=None, propertie
     # the same rows read through the reversed-edge map for the grouping by source atom (no counting pass, no sort); a
     # list that outgrew its capacity exposes empty segments
     rev = torch.zeros(nl.cap_edges if static else max(nl.n_edges, 1), dtype=torch.int32, device=dev)
-    L.check(L.load().nn_nbr_edge_reverse(C.byref(nl.struct), rev.data_ptr(), _stream()), 'nn_nbr_edge_reverse')
+    L.check(L.load().nn_nbr_edge_reverse(C.byref(nl.struct), rev.data_ptr(), stream()), 'nn_nbr_edge_reverse')
     row_ptr = torch.where(nl.status[L.ST_EDGE_OVERFLOW] != 0, torch.zeros_like(nl.row_ptr), nl.row_ptr)
     seg_dst = Segments.from_csr(dst, N, row_ptr)
     seg_src = Segments.from_csr(src, N, row_ptr, perm=rev)
@@ -971,9 +967,10 @@ class GraphedTrainingStep:
     before it goes on - parameters are the same as with the strict path; only the loss RETURNED by the overflowing call
     is that of the empty padded graph.  Any other optimizer (or deferred_check=False) reads the flag every step."""
 
+    HEADROOM = (1.05, 256)         # tight edge capacity: factor and slack over the counted edges
+
     def __init__(self, model, optimizer, z, pos, cell, batch, e_target, f_target, force_weight=50.0, clip_grad=1.0,
                  group=None, cap_edges=None, regrow=True, deferred_check=True):
-        from newtonnet_b200.engine import get_engine
         dev = pos.device
         self.model, self.optimizer, self.group = model, optimizer, group
         self.force_weight, self.clip_grad, self.regrow = float(force_weight), clip_grad, bool(regrow)
@@ -982,7 +979,6 @@ class GraphedTrainingStep:
         self.cell = cell.detach().clone().to(torch.float32).reshape(-1, 3, 3).contiguous()
         self.e_target, self.f_target = e_target.detach().clone(), f_target.detach().clone()
         self.engine = get_engine(dev)
-        self.lib = L.load()
         self.sink = weight_grad_sink(dev)
         self.recaptures = 0
         self.deferred_check = bool(deferred_check)
@@ -990,45 +986,31 @@ class GraphedTrainingStep:
         self._flag_host = torch.zeros(1, dtype=torch.float32).pin_memory()
         self._flag_event = torch.cuda.Event()
         if cap_edges is None:
-            probe = self.engine.neighbor_list(self.pos, self.cell, self.batch, model.cutoff)
-            cap_edges = self._headroom(int(probe.check()[L.ST_N_EDGES]))
+            cap_edges = self._capacity(count_edges(self.engine, self.pos, self.cell, self.batch, model.cutoff).n_edges)
+        else:
+            cap_edges = edge_capacity(cap_edges, 1, 0)      # a given capacity is only made even
         self._capture(cap_edges)
         self.replays = 0
 
-    def _headroom(self, n_edges):
-        cap = int(n_edges * 1.05) + 256
-        if bool((self.cell == 0).all()):                    # non-periodic: all ordered pairs within a molecule bound the list
-            n = torch.bincount(self.batch, minlength=self.cell.shape[0])
-            cap = min(cap, int((n * (n - 1)).sum().item()))
-        return cap
+    def _capacity(self, n_edges):
+        return edge_capacity(n_edges, *self.HEADROOM, all_pairs_bound(self.cell, self.batch))
 
     def _capture(self, cap_edges):
-        from newtonnet_b200.engine import NeighborList
         dev = self.pos.device
-        cap_edges = max(int(cap_edges) + int(cap_edges) % 2, 2)
         self.graph = None                                   # a previous capture's memory pool goes first
         self.nl = NeighborList(self.engine, self.pos, self.cell, self.batch, cap_edges=cap_edges)
         self.model.train()
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):                       # warm-up on a side stream, as graph capture requires
-            for _ in range(2):
-                self.optimizer.zero_grad(set_to_none=True)
-                self._forward_backward()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        torch.cuda.synchronize(dev)
+
+        def zeroed_step():
+            self.optimizer.zero_grad(set_to_none=True)
+            self._forward_backward()
+        warm_up(zeroed_step, dev, 2)
         self.optimizer.zero_grad(set_to_none=True)
-        graph = torch.cuda.CUDAGraph()
-        self.lib.nn_launch_count(1)
-        with torch.cuda.graph(graph):
-            self.loss = self._forward_backward()
-        self.graph = graph
-        self.kernels_per_replay = int(self.lib.nn_launch_count(0))      # this library's kernels recorded in the graph
+        # kernels_per_replay: this library's kernels recorded in the graph
+        self.graph, self.loss, self.kernels_per_replay = capture(self._forward_backward, dev)
 
     def _forward_backward(self):
-        s = _stream()
-        L.check(self.lib.nn_nbr_count(C.byref(self.nl.struct), self.model.cutoff, s), 'nn_nbr_count')
-        L.check(self.lib.nn_nbr_fill(C.byref(self.nl.struct), self.model.cutoff, s), 'nn_nbr_fill')
+        self.nl.rebuild(self.model.cutoff)
         pos = self.pos.clone().requires_grad_(True)
         out = differentiable_forward(self.model, self.z, pos, self.cell, self.batch, static_nl=self.nl)
         loss = Fn.mse_loss(out.energy, self.e_target) + self.force_weight * Fn.mse_loss(out.gradient_force, self.f_target)
@@ -1076,7 +1058,7 @@ class GraphedTrainingStep:
                 raise RuntimeError(f'edge capacity {self.nl.cap_edges} of the captured training graph overflowed on some rank '
                                    f'(this rank needs {need}): the step was NOT applied; rebuild GraphedTrainingStep with a larger cap_edges')
             if need:                             # this rank re-captures with room for the batch that did not fit; all ranks run the step again
-                self._capture(max(self._headroom(need), self.nl.cap_edges + 2))
+                self._capture(max(self._capacity(need), self.nl.cap_edges + 2))
                 self.recaptures += 1
         self._apply()
 

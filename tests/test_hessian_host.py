@@ -109,16 +109,3 @@ def test_bad_selection():
     with pytest.raises(ValueError):
         plan_passes([3, 4], atoms=[])
 
-
-def test_gc_paused_restores_the_collector_state():
-    import gc
-    from newtonnet_b200.hessian import _gc_paused
-    was = gc.isenabled()
-    try:
-        for before in (True, False):
-            (gc.enable if before else gc.disable)()
-            with _gc_paused():
-                assert not gc.isenabled()
-            assert gc.isenabled() == before
-    finally:
-        (gc.enable if was else gc.disable)()
