@@ -473,6 +473,31 @@ NN_API int nn_md_advance(int32_t n_atoms, double* x, double* v, const float* for
 NN_API int nn_md_finish(int32_t n_systems, const int32_t* sys_ptr, double* v, const float* force, const double* inv_mass,
                         double dt, const float* energy, double* log, int32_t log_cap, int64_t* step_ctr,
                         const int32_t* nbr_status, int32_t* sticky, uint32_t* ticket, void* stream);
+/* pos_model = x wrapped into each atom's cell, in fp32 (the wrap nn_md_advance and nn_fire_step apply after a step). */
+NN_API int nn_wrap_positions(int32_t n_atoms, const double* x, const float* cell, const int64_t* batch, float* pos_model,
+                             void* stream);
+
+/* ---- device-resident geometry optimisation: FIRE per system of a batch (newtonnet_b200/optimize.py) ---------------
+ * Replaces the host loop of an ASE optimiser around MLAseCalculator.calculate (utils/ase_interface.py:52-81): one step =
+ * nn_fire_step -> nn_nbr_count -> nn_nbr_fill -> nn_eval -> nn_fire_check, capturable as one CUDA graph (all per-system
+ * state, fmax and the step counter live in device memory).  The step is ase.optimize.FIRE.step (ASE 3.22 / 3.23,
+ * downhill_check=False, no masses, ASE time units) run independently for every system b = [sys_ptr[b], sys_ptr[b+1]).
+ * x, v: [n_atoms,3] fp64 (x unwrapped); force: [n_atoms,3] fp32 at x; pos_model: [n_atoms,3] fp32 wrapped, bound to
+ * nn_nbr.pos; cell: [n_systems,3,3] (all zero = not periodic).
+ * sys_f64: [n_systems,3] {dt, a, max_i |f_i|^2}; sys_i32: [n_systems,4] {Nsteps, started, converged, steps taken}.
+ * Every sum is a fixed-order reduction over the system's own atoms, so a system's trajectory does not depend on which
+ * other systems share the batch.  A converged system is not touched (its x, v and state are frozen). */
+NN_API int nn_fire_step(int32_t n_systems, const int32_t* sys_ptr, double* x, double* v, const float* force, const float* cell,
+                        float* pos_model, double* sys_f64, int32_t* sys_i32, double maxstep, double dtmax, double finc,
+                        double fdec, double astart, double fa, int32_t nmin, void* stream);
+/* After nn_eval: zeroes the forces of fixed atoms (fixed: [n_atoms] 0/1 bytes, or NULL), stores max_i |f_i|^2 over the
+ * system in fp64 and sets converged = (max_i |f_i|^2 < *fmax2) (ASE's Optimizer.converged).  advance != 0 (the captured
+ * step): also counts one step for every system that was not converged before the call, ORs the neighbour-list status words
+ * into sticky[0..2] = {edges needed, max degree, singular cell} and increments *step_ctr (ticket: one zero-initialised
+ * uint32, returned to 0).  advance = 0 only measures: step_ctr, nbr_status, sticky and ticket may be NULL. */
+NN_API int nn_fire_check(int32_t n_systems, const int32_t* sys_ptr, float* force, const uint8_t* fixed, const double* fmax2,
+                         double* sys_f64, int32_t* sys_i32, int32_t advance, int64_t* step_ctr, const int32_t* nbr_status,
+                         int32_t* sticky, uint32_t* ticket, void* stream);
 
 /* ---- Hessian in blocks of rows (newtonnet_b200/hessian.py; reference models/output.py:141-152 batches rows with vmap) ----
  * A pass puts k copies of frames of n_slot atoms into one batch (copy c = system c) and differentiates <seed, pos_grad>

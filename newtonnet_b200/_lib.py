@@ -134,6 +134,10 @@ SYMBOLS = {
     'nn_node_aggregate_bwd': (C.c_int, [C.POINTER(Nbr), _fp, _fp, _fp, _fp, _fp, _fp, _fp]),
     'nn_md_advance': (C.c_int, [C.c_int32, _fp, _fp, _fp, _fp, _fp, _fp, _fp, C.c_double, C.c_double, C.c_double, C.c_uint64, _fp, _fp]),
     'nn_md_finish': (C.c_int, [C.c_int32, _fp, _fp, _fp, _fp, C.c_double, _fp, _fp, C.c_int32, _fp, _fp, _fp, _fp, _fp]),
+    'nn_wrap_positions': (C.c_int, [C.c_int32, _fp, _fp, _fp, _fp, _fp]),
+    'nn_fire_step': (C.c_int, [C.c_int32, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, C.c_double, C.c_double, C.c_double,
+                               C.c_double, C.c_double, C.c_double, C.c_int32, _fp]),
+    'nn_fire_check': (C.c_int, [C.c_int32, _fp, _fp, _fp, _fp, _fp, _fp, C.c_int32, _fp, _fp, _fp, _fp, _fp]),
     'nn_edge_geom_fwd': (C.c_int, [_fp, _fp, C.c_float, _fp, C.c_int32, _fp, _fp, _fp, _fp, _fp]),
     'nn_edge_geom_bwd': (C.c_int, [_fp, C.c_int32, _fp, _fp, _fp, C.c_float, _fp, C.c_int32, _fp, _fp]),
     'nn_message_prepare_b': (C.c_int, [_fp, _fp, _fp]),

@@ -7,6 +7,7 @@ import ctypes as C
 import gc
 import os
 
+import numpy as np
 import torch
 
 from . import _lib as L
@@ -294,6 +295,74 @@ def warm_up(fn, device, times):
         for _ in range(times):
             fn()
     torch.cuda.current_stream(device).wait_stream(side)
+
+
+def driver_inputs(model, z, pos, cell, batch, who):
+    """Inputs of a device-resident driver (DeviceMD, DeviceFIRE), on the model's CUDA device.  Returns (device, engine,
+    weight pack, as_t, z [N] int64, x [N,3] fp64 (a copy), batch [N] int64, cell [B,3,3] fp32); as_t(array, dtype)
+    moves one more input there.  cell None = not periodic, batch None = one system."""
+    dev = next(model.parameters()).device
+    if dev.type != 'cuda':
+        raise RuntimeError(f'{who} needs the model on a CUDA device (no CPU fallback)')
+    as_t = lambda a, dt: torch.as_tensor(np.asarray(a) if not torch.is_tensor(a) else a).to(device=dev, dtype=dt).contiguous()
+    z = as_t(z, torch.int64)
+    N = z.shape[0]
+    x = as_t(pos, torch.float64).reshape(N, 3).clone()
+    batch = torch.zeros(N, dtype=torch.int64, device=dev) if batch is None else as_t(batch, torch.int64)
+    B = int(batch.max().item()) + 1 if N else 1
+    cell = torch.zeros(B, 3, 3, dtype=torch.float32, device=dev) if cell is None else as_t(cell, torch.float32).reshape(-1, 3, 3)
+    if cell.shape[0] != B:
+        raise ValueError(f'cell has {cell.shape[0]} systems, batch has {B}')
+    return dev, get_engine(dev), model._weight_pack(dev), as_t, z, x, batch, cell
+
+
+class ForceStep:
+    """Energy + forces of a device-resident driver's fixed buffers: a neighbour list over (pos, cell, batch) with room for
+    the edges counted plus `headroom`, nn_eval's workspace and arguments.  Calling it rebuilds the list and evaluates, on
+    the current stream and capturable.  Use `force_step` to get one that holds every edge."""
+
+    def __init__(self, engine, weights, z, pos, cell, batch, energy, force, n_edges, headroom):
+        self.engine, self.weights = engine, weights
+        self.nl = NeighborList(engine, pos, cell, batch, cap_edges=edge_capacity(n_edges, *headroom))
+        nbytes = engine.lib.nn_eval_workspace_bytes(self.nl.n_atoms, self.nl.n_systems, self.nl.cap_pairs, weights.n_layers, 1)
+        self.ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=pos.device)
+        self.args = eval_args(self.nl, weights, z, {'energy': energy, 'forces': force}, self.ws, True, False)
+
+    def __call__(self):
+        self.nl.rebuild(self.weights.cutoff)
+        L.check(self.engine.lib.nn_eval(C.byref(self.args), stream()), 'nn_eval')
+
+
+def force_step(engine, weights, z, pos, cell, batch, energy, force, n_edges, headroom):
+    """A ForceStep for `n_edges` edges that has evaluated energy and forces at the current positions, regrown until its
+    neighbour list holds every edge."""
+    while True:
+        fs = ForceStep(engine, weights, z, pos, cell, batch, energy, force, n_edges, headroom)
+        fs()
+        st = fs.nl.check()
+        if not st[L.ST_EDGE_OVERFLOW]:
+            return fs
+        n_edges = edges_needed(st)
+
+
+def replay_chunk(graph, n, sticky, state):
+    """Replay a device-resident driver's step graph n times, then read its sticky status words {edges needed, max degree,
+    singular cell} once (synchronises).  Raises on a singular cell or an over-full row.  Returns 0, or after a capacity
+    overflow somewhere in the chunk the edges a list must hold: every tensor of `state` is then back at its value before
+    the chunk and `sticky` is cleared, so the caller regrows and redoes the chunk."""
+    snap = [t.clone() for t in state]
+    for _ in range(n):
+        graph.replay()
+    st = sticky.cpu().tolist()
+    if st[2]:
+        raise RuntimeError('singular cell in a periodic system')
+    if st[1]:
+        raise RuntimeError(f'an atom has {st[1]} neighbours (> 512)')
+    if st[0]:
+        for t, s in zip(state, snap):
+            t.copy_(s)
+        sticky.zero_()
+    return st[0]
 
 
 class Engine:

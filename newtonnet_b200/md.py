@@ -12,14 +12,13 @@ comparable step by step anyway, so parity is (a) NVE trajectories against a host
 the calculator and (b) the thermostat's temperature.  Units are ASE's: Angstrom, eV, amu, time in
 Angstrom*sqrt(amu/eV) (`FS` converts femtoseconds), `KB` in eV/K.
 """
-import ctypes as C
 import math
 
 import numpy as np
 import torch
 
 from newtonnet_b200 import _lib as L
-from newtonnet_b200.engine import NeighborList, capture, count_edges, edge_capacity, edges_needed, eval_args, get_engine, stream
+from newtonnet_b200.engine import capture, count_edges, driver_inputs, force_step, replay_chunk, stream
 
 __all__ = ['DeviceMD', 'FS', 'KB', 'ATOMIC_MASSES']
 
@@ -29,6 +28,13 @@ ATOMIC_MASSES = np.array([0.0, 1.008, 4.002602, 6.94, 9.0121831, 10.81, 12.011, 
                           22.98976928, 24.305, 26.9815385, 28.085, 30.973761998, 32.06, 35.45, 39.948, 39.0983, 40.078,
                           44.955908, 47.867, 50.9415, 51.9961, 54.938044, 55.845, 58.933194, 58.6934, 63.546, 65.38,
                           69.723, 72.630, 74.921595, 78.971, 79.904, 83.798])
+
+
+def atoms_cell(atoms):
+    """[3,3] fp64 cell of an ASE-like Atoms with the rows of non-periodic directions zeroed (ase_interface.py:134-138)."""
+    cell = np.array(getattr(atoms.get_cell(), 'array', atoms.get_cell()), dtype=np.float64).reshape(3, 3)
+    cell[~np.asarray(atoms.get_pbc(), dtype=bool).reshape(3)] = 0.0
+    return cell
 
 
 class DeviceMD:
@@ -44,21 +50,10 @@ class DeviceMD:
     def __init__(self, model, z, pos, cell=None, batch=None, masses=None, timestep=0.5 * FS, temperature_K=None,
                  friction=None, velocities=None, seed=0, log_capacity=1024, check_interval=64):
         self.lib = L.load()
-        dev = next(model.parameters()).device
-        if dev.type != 'cuda':
-            raise RuntimeError('DeviceMD needs the model on a CUDA device (no CPU fallback)')
-        self.device, self.model = dev, model
-        self.engine = get_engine(dev)
-        self.weights = model._weight_pack(dev)
-        as_t = lambda a, dt: torch.as_tensor(np.asarray(a) if not torch.is_tensor(a) else a).to(device=dev, dtype=dt).contiguous()
-        self.z = as_t(z, torch.int64)
-        N = self.z.shape[0]
-        self.x = as_t(pos, torch.float64).reshape(N, 3).clone()
-        self.batch = torch.zeros(N, dtype=torch.int64, device=dev) if batch is None else as_t(batch, torch.int64)
-        B = int(self.batch.max().item()) + 1 if N else 1
-        self.cell = torch.zeros(B, 3, 3, dtype=torch.float32, device=dev) if cell is None else as_t(cell, torch.float32).reshape(-1, 3, 3)
-        if self.cell.shape[0] != B:
-            raise ValueError(f'cell has {self.cell.shape[0]} systems, batch has {B}')
+        self.model = model
+        dev, self.engine, self.weights, as_t, self.z, self.x, self.batch, self.cell = driver_inputs(model, z, pos, cell, batch, 'DeviceMD')
+        self.device = dev
+        N, B = self.z.shape[0], self.cell.shape[0]
         if masses is None:
             zc = self.z.cpu().numpy()
             if zc.max() >= len(ATOMIC_MASSES):
@@ -96,14 +91,12 @@ class DeviceMD:
     @classmethod
     def from_atoms(cls, atoms, calc, **kwargs):
         """From an ASE-like Atoms object and an MLAseCalculator (scripts/simulate.py:10-31)."""
-        cell = np.array(getattr(atoms.get_cell(), 'array', atoms.get_cell()), dtype=np.float64).reshape(3, 3)
-        cell[~np.asarray(atoms.get_pbc(), dtype=bool).reshape(3)] = 0.0
         kw = dict(kwargs)
         if hasattr(atoms, 'get_masses'):
             kw.setdefault('masses', atoms.get_masses())
         if hasattr(atoms, 'get_velocities') and atoms.get_velocities() is not None and np.any(atoms.get_velocities()):
             kw.setdefault('velocities', atoms.get_velocities())
-        return cls(calc.model, atoms.get_atomic_numbers(), atoms.get_positions(), cell[None], **kw)
+        return cls(calc.model, atoms.get_atomic_numbers(), atoms.get_positions(), atoms_cell(atoms)[None], **kw)
 
     def update_atoms(self, atoms):
         atoms.set_positions(self.positions)
@@ -118,11 +111,8 @@ class DeviceMD:
                                        stream()), 'nn_md_advance')
 
     def _wrap(self):
-        self._advance(0.0, 1.0)          # zero time step: only writes the wrapped fp32 copy
-
-    def _forces(self):
-        self.nl.rebuild(self.weights.cutoff)
-        L.check(self.lib.nn_eval(C.byref(self.args), stream()), 'nn_eval')
+        L.check(self.lib.nn_wrap_positions(self.n_atoms, self.x.data_ptr(), self.cell.data_ptr(), self.batch.data_ptr(),
+                                           self.pos_model.data_ptr(), stream()), 'nn_wrap_positions')
 
     def _finish(self):
         L.check(self.lib.nn_md_finish(self.n_systems, self.nl.sys_ptr.data_ptr(), self.v.data_ptr(), self.force.data_ptr(),
@@ -132,19 +122,14 @@ class DeviceMD:
 
     def _step(self):
         self._advance(self.dt, self.ou_c)
-        self._forces()
+        self.forces_step()
         self._finish()
 
     def _build(self, n_edges):
         """(Re)allocate the neighbour list for `n_edges`, evaluate forces at the current positions and capture the step."""
-        self.nl = NeighborList(self.engine, self.pos_model, self.cell, self.batch, cap_edges=edge_capacity(n_edges, *self.HEADROOM))
-        nbytes = self.lib.nn_eval_workspace_bytes(self.n_atoms, self.n_systems, self.nl.cap_pairs, self.weights.n_layers, 1)
-        self.ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-        self.args = eval_args(self.nl, self.weights, self.z, {'energy': self.energy, 'forces': self.force}, self.ws, True, False)
-        self._forces()
-        st = self.nl.check()
-        if st[L.ST_EDGE_OVERFLOW]:
-            return self._build(edges_needed(st))
+        self.forces_step = force_step(self.engine, self.weights, self.z, self.pos_model, self.cell, self.batch, self.energy,
+                                      self.force, n_edges, self.HEADROOM)
+        self.nl = self.forces_step.nl
         self.graph, _, self.kernels_per_step = capture(self._step, self.device)     # kernels one graph replay launches
 
     # ------------------------------------------------------------------ run
@@ -159,21 +144,12 @@ class DeviceMD:
             n = min(self.check_interval, steps - done)
             if trajectory_interval:
                 n = min(n, trajectory_interval - (done % trajectory_interval))
-            snap = (self.x.clone(), self.v.clone(), self.force.clone(), self.step_ctr.clone())
-            s0 = int(snap[3].item())
-            for _ in range(n):
-                self.graph.replay()
+            s0 = self.step
+            need = replay_chunk(self.graph, n, self.sticky, (self.x, self.v, self.force, self.step_ctr))
             self.graph_launches += n
-            sticky = self.sticky.cpu().tolist()                # one D2H read per chunk (synchronises)
-            if sticky[2]:
-                raise RuntimeError('singular cell in a periodic system')
-            if sticky[1]:
-                raise RuntimeError(f'an atom has {sticky[1]} neighbours (> 512)')
-            if sticky[0]:                                      # capacity overflow somewhere in the chunk: roll back, regrow, redo
-                self.x.copy_(snap[0]); self.v.copy_(snap[1]); self.force.copy_(snap[2]); self.step_ctr.copy_(snap[3])
-                self.sticky.zero_()
+            if need:                                           # capacity overflow somewhere in the chunk: rolled back; regrow, redo
                 self._wrap()
-                self._build(sticky[0])
+                self._build(need)
                 continue
             rows = (torch.arange(s0, s0 + n, device=self.device) % self.log_capacity)
             chunk = self.log[rows].cpu().numpy()
