@@ -499,6 +499,27 @@ NN_API int nn_fire_check(int32_t n_systems, const int32_t* sys_ptr, float* force
                          double* sys_f64, int32_t* sys_i32, int32_t advance, int64_t* step_ctr, const int32_t* nbr_status,
                          int32_t* sticky, uint32_t* ticket, void* stream);
 
+/* ---- device-resident climbing-image NEB: one FIRE system per band (newtonnet_b200/neb.py) ------------------------------
+ * One step = nn_fire_step (band ranges) -> nn_nbr_count -> nn_nbr_fill -> nn_eval (one system per interior image) ->
+ * nn_neb_forces -> nn_fire_check (band ranges, on neb_force), capturable as one CUDA graph.
+ * NEB force of every interior image: ASE's NEB.get_forces with method='improvedtangent' and a scalar spring constant k
+ * (ASE 3.22; where an image and both neighbours have equal energies the tangent is t+ + t-, not ASE's zero vector).
+ * One block per interior image j of n_images; bands are stored band-major and images image-major:
+ * img_ptr [n_images+1] first atom of each interior image; img_band [n_images] its band; band_img [n_bands+1] first
+ * interior image of each band.  x [*,3] fp64 positions of the interior images; ends [*,3] fp64 end-point positions:
+ * band b's image 0 at rows band_ends[b].., its last image right after; energy [n_images] fp32 (nn_eval's output);
+ * ends_energy [n_bands,2] fp64; force [*,3] fp32 model forces (fixed: 0/1 bytes or NULL, fixed atoms' forces count as 0).
+ * climb [n_bands] 0/1: the highest interior image (ties to the highest index) climbs; imax [n_bands] receives its index in
+ * 1..n.  band_si: nn_fire_step's per-band int32 state: the blocks of a converged band write nothing.
+ * neb_force [*,3] fp32 receives the NEB force (0 for fixed atoms).  A band whose model output is not finite (an interior
+ * energy, or a force of a free atom) gets a zero NEB force on every image and failed[b] = 1 (failed: [n_bands] int32, only
+ * ever set), so nn_fire_check finds it converged and the FIRE kernels leave it at its last, finite positions.  Spring vectors are never wrapped: periodic images
+ * must be aligned (minimum-image displacements between consecutive images) before they are passed in. */
+NN_API int nn_neb_forces(int32_t n_images, const int32_t* img_ptr, const int32_t* img_band, const int32_t* band_img,
+                         const double* x, const double* ends, const int32_t* band_ends, const float* energy,
+                         const double* ends_energy, const float* force, const uint8_t* fixed, const int32_t* climb,
+                         const int32_t* band_si, double k, float* neb_force, int32_t* imax, int32_t* failed, void* stream);
+
 /* ---- Hessian in blocks of rows (newtonnet_b200/hessian.py; reference models/output.py:141-152 batches rows with vmap) ----
  * A pass puts k copies of frames of n_slot atoms into one batch (copy c = system c) and differentiates <seed, pos_grad>
  * once: copy c's block of that gradient is row plan[pass][c].row of its frame's Hessian.

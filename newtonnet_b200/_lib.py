@@ -138,6 +138,8 @@ SYMBOLS = {
     'nn_fire_step': (C.c_int, [C.c_int32, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, C.c_double, C.c_double, C.c_double,
                                C.c_double, C.c_double, C.c_double, C.c_int32, _fp]),
     'nn_fire_check': (C.c_int, [C.c_int32, _fp, _fp, _fp, _fp, _fp, _fp, C.c_int32, _fp, _fp, _fp, _fp, _fp]),
+    'nn_neb_forces': (C.c_int, [C.c_int32, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, C.c_double, _fp, _fp,
+                                _fp, _fp]),
     'nn_edge_geom_fwd': (C.c_int, [_fp, _fp, C.c_float, _fp, C.c_int32, _fp, _fp, _fp, _fp, _fp]),
     'nn_edge_geom_bwd': (C.c_int, [_fp, C.c_int32, _fp, _fp, _fp, C.c_float, _fp, C.c_int32, _fp, _fp]),
     'nn_message_prepare_b': (C.c_int, [_fp, _fp, _fp]),

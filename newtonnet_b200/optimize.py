@@ -27,6 +27,37 @@ DT, A, F2 = 0, 1, 2
 NSTEPS, STARTED, CONVERGED, STEPS = 0, 1, 2, 3
 
 
+def segment_rows(ptr, sel):
+    """Row indices of segments `sel` (ascending) of an array cut at offsets `ptr`: rows [ptr[s], ptr[s+1]) of every s in
+    sel, in order.  The rows a step graph gathers for the systems it keeps."""
+    ptr, sel = np.asarray(ptr, dtype=np.int64), np.asarray(sel, dtype=np.int64)
+    n = ptr[sel + 1] - ptr[sel]
+    return np.repeat(ptr[sel], n) + np.arange(int(n.sum())) - np.repeat(np.cumsum(n) - n, n)
+
+
+def gather_state(w, master, index, keys):
+    """w.<key> = master[key][index] as a fresh contiguous tensor, for every key."""
+    for k in keys:
+        setattr(w, k, master[k][index].contiguous())
+
+
+def scatter_state(master, w, index, keys):
+    """master[key][index] = w.<key>, for every key: the inverse of gather_state."""
+    for k in keys:
+        master[k].index_copy_(0, index, getattr(w, k))
+
+
+def fixed_mask(atoms, who):
+    """[len(atoms)] bool: the atoms FixAtoms-like constraints (any object with get_indices()) hold in place.  Any other
+    constraint raises NotImplementedError."""
+    f = np.zeros(len(atoms), dtype=bool)
+    for c in getattr(atoms, 'constraints', None) or ():
+        if not hasattr(c, 'get_indices'):
+            raise NotImplementedError(f'{who} supports FixAtoms-like constraints only, not {type(c).__name__}')
+        f[np.asarray(c.get_indices(), dtype=np.int64)] = True
+    return f
+
+
 def compaction_plan(active, n_atoms):
     """Which systems a relaxation keeps in its step graph at a chunk boundary.  active: bool [S], the systems of the
     graph's batch that have not converged; n_atoms: [S] atoms per system.  Returns None while the active systems hold
@@ -86,14 +117,7 @@ class DeviceFIRE:
         """From one ASE-like Atoms or a list (one system each) and an MLAseCalculator.  FixAtoms-like constraints (any
         object with get_indices()) become `fixed`; any other constraint raises NotImplementedError."""
         atoms_list = cls._atoms_list(atoms)
-        fixed = []
-        for at in atoms_list:
-            f = np.zeros(len(at), dtype=bool)
-            for c in getattr(at, 'constraints', None) or ():
-                if not hasattr(c, 'get_indices'):
-                    raise NotImplementedError(f'DeviceFIRE supports FixAtoms-like constraints only, not {type(c).__name__}')
-                f[np.asarray(c.get_indices(), dtype=np.int64)] = True
-            fixed.append(f)
+        fixed = [fixed_mask(at, 'DeviceFIRE') for at in atoms_list]
         kw = dict(kwargs)
         if any(f.any() for f in fixed):
             kw.setdefault('fixed', np.concatenate(fixed))
@@ -113,14 +137,12 @@ class DeviceFIRE:
         """Point the step graph at master systems `sel` (ascending) with atom system ids `batch`: gather their state into
         fresh buffers, evaluate and capture."""
         m, dev = self.master, self.device
-        n = self.sys_atoms[sel]
-        atoms = np.repeat(self.sys_ptr[sel], n) + np.arange(int(n.sum())) - np.repeat(np.cumsum(n) - n, n)
+        atoms = segment_rows(self.sys_ptr, sel)
         ai, si = torch.as_tensor(atoms, device=dev), torch.as_tensor(sel, device=dev)
-        w = types.SimpleNamespace(sel=np.asarray(sel), sys_atoms=n, atoms=ai, sys=si, n_atoms=len(atoms), n_systems=len(sel))
-        for k in ('z', 'x', 'v', 'force', 'fixed'):
-            setattr(w, k, m[k][ai].contiguous())
-        for k in ('energy', 'cell', 'sf', 'si'):
-            setattr(w, k, m[k][si].contiguous())
+        w = types.SimpleNamespace(sel=np.asarray(sel), sys_atoms=self.sys_atoms[sel], atoms=ai, sys=si, n_atoms=len(atoms),
+                                  n_systems=len(sel))
+        gather_state(w, m, ai, ('z', 'x', 'v', 'force', 'fixed'))
+        gather_state(w, m, si, ('energy', 'cell', 'sf', 'si'))
         w.batch = torch.as_tensor(batch, dtype=torch.int64, device=dev)
         w.pos_model = torch.empty(len(atoms), 3, dtype=torch.float32, device=dev)
         w.step_ctr = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -133,10 +155,8 @@ class DeviceFIRE:
     def _scatter(self):
         """Copy the graph's systems back into the master state."""
         w, m = self.work, self.master
-        for k in ('x', 'v', 'force'):
-            m[k].index_copy_(0, w.atoms, getattr(w, k))
-        for k in ('energy', 'sf', 'si'):
-            m[k].index_copy_(0, w.sys, getattr(w, k))
+        scatter_state(m, w, w.atoms, ('x', 'v', 'force'))
+        scatter_state(m, w, w.sys, ('energy', 'sf', 'si'))
 
     def _wrap(self):
         w = self.work
