@@ -175,7 +175,6 @@ typedef struct {
     int32_t m;
     int32_t prologue, epilogue;
     int32_t aux_tiled;              /* NN_EPI_MUL only: aux1 is stored tile-transposed (NN_TILED_INDEX), as the chained kernel writes it */
-    int32_t xy_tiled;               /* bit 0: X is tile-transposed (NN_PRO_NONE + NN_EPI_BIAS); bit 1: Y is (NN_EPI_MUL with aux_tiled) */
 } nn_gemm_args;
 /* Tile-transposed ("row-owner") layout of an [M,128] fp32 tensor: tiles of 128 rows, inside a tile the 16-byte chunk c
  * (0..31) of row r (0..127) lives at float offset ((tile * 32 + c) * 128 + r) * 4.  tcgen05.ld / st hand every lane one ROW
@@ -190,7 +189,9 @@ NN_API int nn_gemm128(const nn_gemm_args* a, void* stream);
  *   mid = NN_MID_SILU_SAVE: q = acc + bias1; aux_out = silu'(q); h = silu(q)      (forward)
  *   mid = NN_MID_MUL      : h = acc * aux1                                         (reverse)
  *   out = NN_OUT_BIAS     : Y = acc + bias2 (bias2 may be NULL)     out = NN_OUT_ADD: Y = acc + aux2
- * Bit-identical to two nn_gemm128 calls.  B1_img / B2_img: nn_gemm128_prepare_b images.  tcgen05 only. */
+ * aux_out (mid = SILU_SAVE) and aux1 (mid = MUL) are in the tile-transposed layout (NN_TILED_INDEX) and hold whole tiles
+ * of 128 rows; X, Y and aux2 are row-major.  Bit-identical to two nn_gemm128 calls (the second of a reverse pair reading
+ * aux1 with aux_tiled = 1).  B1_img / B2_img: nn_gemm128_prepare_b images.  tcgen05 only. */
 #define NN_MID_SILU_SAVE 0
 #define NN_MID_MUL 1
 #define NN_OUT_BIAS 0
@@ -208,7 +209,6 @@ typedef struct {
      * in lockstep, so X is fetched from HBM once (the second read is an L2 hit): equiv_message1 and equiv_message2 of one
      * layer share their input (models/newtonnet.py:218,222). */
     const float* B1_img_b; const float* B2_img_b; float* aux_out_b; float* Y_b;
-    int32_t aux_tiled;              /* aux_out (mid = SILU_SAVE) / aux1 (mid = MUL) are in the tile-transposed layout (NN_TILED_INDEX) */
     int32_t pad_;
 } nn_gemm_chain_args;
 NN_API int nn_gemm128_chain(const nn_gemm_chain_args* a, void* stream);
@@ -439,8 +439,7 @@ NN_API int nn_ew_silu(int32_t mode, const float* x, const float* a, const float*
 NN_API int nn_mlp_mid_tiled(int32_t m, int32_t has_m_dev);
 NN_API int nn_mlp_fwd(const float* X, const nn_mat* M1, const float* b1, float* mid, const nn_mat* M2, const float* b2, float* Y,
                       int32_t m, const int32_t* m_dev, int32_t save_dact, void* stream);
-/* Y (+)= ((G M2) * dact) M1: the transpose of nn_mlp_fwd with respect to X.  `tmp` may alias G; like `mid` it holds
- * ceil(m / 128) * 128 rows (the intermediate may travel tile-transposed). */
+/* Y (+)= ((G M2) * dact) M1: the transpose of nn_mlp_fwd with respect to X.  `tmp` [m,128] may alias G. */
 NN_API int nn_mlp_bwd(const float* G, const nn_mat* M2, const float* dact, float* tmp, const nn_mat* M1, float* Y, int32_t m,
                       const int32_t* m_dev, int32_t accumulate, void* stream);
 /* gh2[i,:] = scale[z_i] * w3 * silu'(h2pre[i,:]): d(sum of atomic energies)/d(second hidden layer), models/output.py:98-100 */

@@ -55,13 +55,13 @@ class Nbr(C.Structure):
 class GemmArgs(C.Structure):
     _fields_ = [('X', _fp), ('B', _fp), ('Y', _fp), ('B_img', _fp), ('bias', _fp), ('aux1', _fp), ('aux2', _fp), ('aux3', _fp), ('aux_out', _fp),
                 ('m_dev', _fp), ('m_dev_mul', C.c_int32), ('m', C.c_int32), ('prologue', C.c_int32),
-                ('epilogue', C.c_int32), ('aux_tiled', C.c_int32), ('xy_tiled', C.c_int32)]
+                ('epilogue', C.c_int32), ('aux_tiled', C.c_int32)]
 
 
 class GemmChainArgs(C.Structure):
     _fields_ = [('X', _fp), ('B1_img', _fp), ('B2_img', _fp), ('bias1', _fp), ('bias2', _fp), ('aux1', _fp), ('aux2', _fp),
                 ('aux_out', _fp), ('Y', _fp), ('m_dev', _fp), ('m_dev_mul', C.c_int32), ('m', C.c_int32), ('mid', C.c_int32),
-                ('out', C.c_int32), ('B1_img_b', _fp), ('B2_img_b', _fp), ('aux_out_b', _fp), ('Y_b', _fp), ('aux_tiled', C.c_int32),
+                ('out', C.c_int32), ('B1_img_b', _fp), ('B2_img_b', _fp), ('aux_out_b', _fp), ('Y_b', _fp),
                 ('pad_', C.c_int32)]
 
 

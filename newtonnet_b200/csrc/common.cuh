@@ -11,7 +11,6 @@ static constexpr int kNB = NN_NB;    // 20 radial basis functions
 
 void nn_set_error(const char* fmt, ...);
 bool nn_pdl_enabled();     // programmatic dependent launch of the tensor-core kernels (NN_PDL=0 turns it off)
-bool nn_pdl_all_enabled(); // ... and of the stream kernels too (NN_PDL_ALL=1; off by default, see nn_launch_dep)
 // every kernel launch of this library is counted (bench.py reports it as gpu_launches)
 void nn_count_launches(int n);
 // optional per-stage CUDA-event profiler (nn_profile_enable): stages are timed on the launching stream
@@ -38,32 +37,11 @@ struct ProfScope {
 // first statement of a kernel whose successor may be a PDL kernel (tc_common.cuh): lets that kernel's prologue start
 // as soon as every CTA of this grid is resident; it still waits for this grid to complete before reading its results
 #define NN_PDL_TRIGGER() asm volatile("griddepcontrol.launch_dependents;" ::: "memory")
-// ... and of a kernel that is itself launched as a programmatic dependent (nn_launch_dep): blocks until the preceding
-// grids have completed and their writes are visible; a no-op under a plain launch.  Everything before it may only
-// touch the kernel's own arguments.
-#define NN_PDL_WAIT() asm volatile("griddepcontrol.wait;" ::: "memory")
 
 #define NN_REQUIRE(cond, msg)                                                       \
     do {                                                                            \
         if (!(cond)) { nn_set_error("%s: %s", __func__, msg); return -1; }          \
     } while (0)
-
-// Launch of a stream kernel, optionally (NN_PDL_ALL=1) with the programmatic-stream-serialization attribute like the
-// tensor-core kernels (the kernel executes NN_PDL_WAIT() before it reads anything a predecessor wrote).  MEASURED, B200,
-// round 2: no gain for eagerly launched steps (c4 29.26 -> 29.18 ms, c3 1.944 -> 1.946 ms) and a LOSS when the step is
-// replayed as a CUDA graph (c4 end to end 29.4 -> 33.1 ms, c3 2.04 -> 2.26 ms): the small-register stream kernels become
-// co-resident with the persistent GEMM CTAs they depend on and the graph's programmatic edges serialise worse than plain
-// ones.  So the attribute stays off for them; only the tcgen05 kernels (tc_common.cuh: launch_pdl) are dependents.
-template <typename... KArgs, typename... Args>
-static inline void nn_launch_dep(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = nn_pdl_all_enabled() ? 1 : 0;
-    cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
 
 int nn_num_sms();           // multiprocessor count of the current device (cached per device; 148 on B200)
 static inline int nn_ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }

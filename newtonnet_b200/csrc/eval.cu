@@ -54,12 +54,8 @@ static bool chain_enabled() {          // two-CTA chained GEMM pairs (gemm_chain
 }
 
 // node-level MLPs (no device row count) take the chained kernel when they are small enough to be launch-latency-bound:
-// one launch instead of two (measured: see DESIGN.md); 0 = never.  Large node-level inputs stay on two launches.
-static int chain_small_m() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("NN_CHAIN_SMALL_M"); v = e ? atoi(e) : 20000; }
-    return v;
-}
+// one launch instead of two (measured: see DESIGN.md).  Large node-level inputs stay on two launches.
+constexpr int kChainSmallM = 20000;
 
 bool nn_pdl_enabled() {
     static int v = -1;
@@ -78,12 +74,6 @@ int nn_num_sms() {
         sms[dev] = v > 0 ? v : 148;
     }
     return sms[dev];
-}
-
-bool nn_pdl_all_enabled() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("NN_PDL_ALL"); v = (e && e[0] == '1' && nn_pdl_enabled()) ? 1 : 0; }
-    return v == 1;
 }
 
 extern "C" long long nn_launch_count(int reset) {
@@ -145,23 +135,10 @@ extern "C" int nn_get_gemm_backend(void) { return g_backend; }
 // The chained kernel keeps the activation-derivative tensor silu'(q) in the tile-transposed layout (NN_TILED_INDEX), and
 // the reverse MLP (chained or two launches) reads it there.  Writer and reader take the decision from the same predicate:
 // the chained kernel ran in the forward MLP <=> pair-level call (device row count) or a small node-level call.
-static bool tiled_enabled() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("NN_AUX_TILED"); v = (e && e[0] == '0') ? 0 : 1; }
-    return v == 1;
-}
-static bool tmp_tiled_enabled() {
-    static int v = -1;
-    // measured (B200, pair-level contractions per step): c4 11.22 -> 11.52 ms, c2 7.49 -> 7.67 ms with the tiled intermediate:
-    // the register-held row loads of the second launch keep fewer bytes in flight than its cp.async staging - off by default
-    if (v < 0) { const char* e = getenv("NN_TMP_TILED"); v = (e && e[0] == '1') ? 1 : 0; }
-    return v == 1;
-}
-static bool chain_runs_fwd(const int* m_dev, int m) { return g_backend == 2 && chain_enabled() && (m_dev || m <= chain_small_m()); }
-static bool aux_is_tiled(const int* m_dev, int m) { return tiled_enabled() && chain_runs_fwd(m_dev, m); }
+static bool chain_runs_fwd(const int* m_dev, int m) { return g_backend == 2 && chain_enabled() && (m_dev || m <= kChainSmallM); }
 extern "C" int nn_mlp_mid_tiled(int32_t m, int32_t has_m_dev) {
     static const int one = 1;
-    return aux_is_tiled(has_m_dev ? &one : nullptr, m) ? 1 : 0;
+    return chain_runs_fwd(has_m_dev ? &one : nullptr, m) ? 1 : 0;
 }
 
 
@@ -209,7 +186,7 @@ EvalWs carve_eval(void* base, size_t cap, int N, int B, int P, int L, bool bwd) 
         LayerBuf& b = w.layer[l];
         b.pre = c.take<float>(NFt); b.mn = c.take<float>(NF);
         b.f_out = c.take<float>(3 * NF); b.g = c.take<float>(3 * NF);
-        b.msg = c.take<float>(PF); b.q1 = c.take<float>(PFt); b.e1 = c.take<float>(PFt);      // e1 also hosts the tiled intermediate of the reverse MLP
+        b.msg = c.take<float>(PF); b.q1 = c.take<float>(PFt); b.e1 = c.take<float>(PF);
         if (l > 0) { b.q2 = c.take<float>(PFt); b.e2 = c.take<float>(PF); }
         b.ln_xhat = c.take<float>(NF); b.ln_rstd = c.take<float>(N);
     }
@@ -234,7 +211,6 @@ EvalWs carve_eval(void* base, size_t cap, int N, int B, int P, int L, bool bwd) 
 struct Gemm {
     cudaStream_t s; int rc = 0;
     bool aux_tiled_next = false;          // the next EPI_MUL launch reads its factor in the tile-transposed layout
-    int xy_tiled_next = 0;                // ... and its X (bit 0) / Y (bit 1) are tile-transposed
     // fwd(M): x @ M^T -> B = M.wt ; bwd(M): g @ M -> B = M.w
     void fwd(const float* X, const nn_mat& M, float* Y, int m, int pro, int epi, const float* bias = nullptr,
              const float* aux1 = nullptr, const float* aux2 = nullptr, const float* aux3 = nullptr,
@@ -252,7 +228,6 @@ struct Gemm {
             nn_gemm_chain_args a{};
             a.X = X; a.B1_img = M1.wt_img; a.B2_img = M2.wt_img; a.bias1 = b1; a.bias2 = b2; a.aux_out = mid; a.Y = Y;
             a.m_dev = m_dev; a.m_dev_mul = 1; a.m = m; a.mid = NN_MID_SILU_SAVE; a.out = NN_OUT_BIAS;
-            a.aux_tiled = aux_is_tiled(m_dev, m);
             rc = nn_gemm128_chain(&a, s);
             return;
         }
@@ -263,15 +238,12 @@ struct Gemm {
     bool mlp_fwd_dual(const float* X, const nn_mat& A1, float* midA, const nn_mat& A2, float* YA, const nn_mat& B1, float* midB,
                       const nn_mat& B2, float* YB, int m, const int* m_dev) {
         if (rc) return true;
-        static int dual_on = -1;
-        if (dual_on < 0) { const char* e = getenv("NN_CHAIN_DUAL"); dual_on = (e && e[0] == '0') ? 0 : 1; }
-        if (!(g_backend == 2 && chain_enabled() && dual_on && m_dev && A1.wt_img && A2.wt_img && B1.wt_img && B2.wt_img)) return false;
+        if (!(g_backend == 2 && chain_enabled() && m_dev && A1.wt_img && A2.wt_img && B1.wt_img && B2.wt_img)) return false;
         ProfScope ps(NN_STAGE_PAIR_GEMM, s);
         nn_gemm_chain_args a{};
         a.X = X; a.B1_img = A1.wt_img; a.B2_img = A2.wt_img; a.aux_out = midA; a.Y = YA;
         a.B1_img_b = B1.wt_img; a.B2_img_b = B2.wt_img; a.aux_out_b = midB; a.Y_b = YB;
         a.m_dev = m_dev; a.m_dev_mul = 1; a.m = m; a.mid = NN_MID_SILU_SAVE; a.out = NN_OUT_BIAS;
-        a.aux_tiled = aux_is_tiled(m_dev, m);
         rc = nn_gemm128_chain(&a, s);
         return true;
     }
@@ -279,25 +251,18 @@ struct Gemm {
     void mlp_bwd(const float* G, const nn_mat& M2, const float* dact, float* tmp, const nn_mat& M1, float* Y, int m,
                  bool accumulate, const int* m_dev = nullptr) {
         if (rc) return;
-        if (g_backend == 2 && chain_enabled() && ((m_dev && accumulate) || (!m_dev && m <= chain_small_m())) && M1.w_img && M2.w_img) {
+        if (g_backend == 2 && chain_enabled() && ((m_dev && accumulate) || (!m_dev && m <= kChainSmallM)) && M1.w_img && M2.w_img) {
             ProfScope ps(m_dev ? NN_STAGE_PAIR_GEMM : NN_STAGE_NODE_GEMM, s);
             nn_gemm_chain_args a{};
             a.X = G; a.B1_img = M2.w_img; a.B2_img = M1.w_img; a.aux1 = dact; a.aux2 = accumulate ? Y : nullptr; a.Y = Y;
             a.m_dev = m_dev; a.m_dev_mul = 1; a.m = m; a.mid = NN_MID_MUL; a.out = accumulate ? NN_OUT_ADD : NN_OUT_BIAS;
-            a.aux_tiled = aux_is_tiled(m_dev, m);
             rc = nn_gemm128_chain(&a, s);
             return;
         }
-        // with a tile-transposed silu' the intermediate travels tile-transposed too (pair-level, non-accumulating): the first
-        // launch stores it straight from the tcgen05.ld registers, the second loads it straight into registers
-        aux_tiled_next = aux_is_tiled(m_dev, m);
-        const bool tmp_tiled = aux_tiled_next && m_dev && !accumulate && tmp_tiled_enabled();
-        xy_tiled_next = tmp_tiled ? 2 : 0;
+        aux_tiled_next = chain_runs_fwd(m_dev, m);     // the forward MLP ran chained and left silu' tile-transposed
         bwd(G, M2, tmp, m, NN_PRO_NONE, NN_EPI_MUL, nullptr, dact, nullptr, nullptr, m_dev);
         aux_tiled_next = false;
-        xy_tiled_next = tmp_tiled ? 1 : 0;
         bwd(tmp, M1, Y, m, NN_PRO_NONE, accumulate ? NN_EPI_ADD : NN_EPI_BIAS, nullptr, accumulate ? Y : nullptr, nullptr, nullptr, m_dev);
-        xy_tiled_next = 0;
     }
     void run(const float* X, const float* B, const float* B_img, float* Y, int m, int pro, int epi,
              const float* bias = nullptr, const float* aux1 = nullptr, const float* aux2 = nullptr,
@@ -310,7 +275,6 @@ struct Gemm {
         a.X = X; a.B = B; a.B_img = B_img; a.Y = Y; a.bias = bias; a.aux1 = aux1; a.aux2 = aux2; a.aux3 = aux3;
         a.m_dev = m_dev; a.m_dev_mul = mul; a.m = m; a.prologue = pro; a.epilogue = epi;
         a.aux_tiled = (epi == NN_EPI_MUL && aux_tiled_next) ? 1 : 0;
-        a.xy_tiled = xy_tiled_next;
         rc = nn_gemm128_launch(a, s);
     }
 };

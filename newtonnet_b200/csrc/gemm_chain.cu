@@ -31,7 +31,6 @@
 namespace {
 
 using namespace tc;
-constexpr int NKB = 4;
 constexpr uint32_t B_BYTES = 2 * NKB * BLK_BYTES;     // hi + lo image of one weight matrix = 128 KB
 constexpr uint32_t BAR_BYTES = 512;
 constexpr int PDEPTH = 2;
@@ -97,34 +96,30 @@ struct ChainCtx {
     int warp, lane, cid, ncl, M, my_tiles; bool has_work;
 };
 
-// ===================== epilogue (rank 0: mid step -> peer's ring; rank 1: output step -> Y) =====================
-template <int MID, int OUT, int RANK>
-__device__ __forceinline__ void epilogue_role(const nn_gemm_chain_args& a, const ChainCtx& x) {
-    const uint32_t base = x.base, sPst = x.sPst, sStg = x.sStg, tmem_base = x.tmem_base;
-    const uint32_t bar_t_full = x.bar_t_full, bar_t_empty = x.bar_t_empty, bar_ring_full = x.bar_ring_full,
-                   bar_ring_empty = x.bar_ring_empty;
+// ===================== rank-1 epilogue: output step -> Y =====================
+template <int OUT>
+__device__ __forceinline__ void epilogue_rank1(const nn_gemm_chain_args& a, const ChainCtx& x) {
+    const uint32_t base = x.base, sStg = x.sStg, tmem_base = x.tmem_base;
+    const uint32_t bar_t_full = x.bar_t_full, bar_t_empty = x.bar_t_empty;
     uint8_t* smem_gen = x.smem_gen;
     const int warp = x.warp, lane = x.lane, cid = x.cid, ncl = x.ncl, M = x.M, my_tiles = x.my_tiles;
-    const bool has_work = x.has_work;
-    (void)bar_ring_full; (void)bar_ring_empty; (void)sPst;
     const int q = warp & 3, ew = warp - PRODUCER_WARPS, half = ew >> 2;
     const int r4 = lane >> 3, c8 = lane & 7;
     uint8_t* stg = smem_gen + (sStg - base) + ew * STG_BYTES;
-    // rank 0 writes into rank 1's ring: producer warp (q, half) there owns blocks [PDEPTH] at the same offsets
-    const uint32_t ring_remote = map_to_rank(sPst + (half * 4 + q) * PDEPTH * STG_BYTES, 1);
-    constexpr bool aux_in = (RANK == 0 && MID == MID_MUL) || (RANK == 1 && OUT == OUT_ADD);
-    const float* aux = RANK == 0 ? a.aux1 : a.aux2;
-    const float* bias = RANK == 0 ? a.bias1 : a.bias2;
+    // Rank 1 sends nothing to its peer, so the two peer addresses (ring block, ring_full slot) are unused here.  They are
+    // still computed: mapa is volatile asm, and without it ptxas schedules all four kernel variants differently.
+    (void)map_to_rank(x.sPst + (half * 4 + q) * PDEPTH * STG_BYTES, 1);
+    constexpr bool aux_in = OUT == OUT_ADD;
     float4 ax[8];
     auto prefetch = [&](int tile, int c0) {
         if (!aux_in) return;
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
             const int grow = tile * TM + q * 32 + k * 4 + r4;
-            if (grow < M) ax[k] = ld4(aux + (size_t)grow * 128 + c0 + 4 * c8);
+            if (grow < M) ax[k] = ld4(a.aux2 + (size_t)grow * 128 + c0 + 4 * c8);
         }
     };
-    if (has_work) prefetch(cid, half * 64);
+    if (x.has_work) prefetch(cid, half * 64);
     uint32_t it = 0;
     for (int t = 0; t < my_tiles; ++t, ++it) {
         const int tile = cid + t * ncl;
@@ -158,29 +153,14 @@ __device__ __forceinline__ void epilogue_role(const nn_gemm_chain_args& a, const
             }
             const int col = c0 + 4 * c8;
             float4 bv = f4_zero();
-            if (bias) bv = ld4(bias + col);
-            const uint32_t full_remote = map_to_rank(bar_ring_full + 8 * slot, 1);
-            if (RANK == 0) mbar_wait_cluster(bar_ring_empty + 8 * slot, (t & 1) ^ 1);   // rank 1 has read tile t-1's block
+            if (a.bias2) bv = ld4(a.bias2 + col);
+            (void)map_to_rank(x.bar_ring_full + 8 * slot, 1);
 #pragma unroll
             for (int k = 0; k < 8; ++k) {
                 const int row = k * 4 + r4;
                 const int grow = tile * TM + q * 32 + row;
                 float4 acc = *reinterpret_cast<const float4*>(stg + row * 128 + ((c8 ^ (row & 7)) << 4));
-                if (RANK == 0) {
-                    float4 hmid;
-                    if (MID == MID_SILU_SAVE) {
-                        const float4 x = f4_add(acc, bv);
-                        const float4 s = make_float4(sigmoid_f(x.x), sigmoid_f(x.y), sigmoid_f(x.z), sigmoid_f(x.w));
-                        if (grow < M)
-                            st4(a.aux_out + (size_t)grow * 128 + col,
-                                make_float4(s.x * fmaf(x.x, 1.0f - s.x, 1.0f), s.y * fmaf(x.y, 1.0f - s.y, 1.0f),
-                                            s.z * fmaf(x.z, 1.0f - s.z, 1.0f), s.w * fmaf(x.w, 1.0f - s.w, 1.0f)));
-                        hmid = f4_mul(x, s);
-                    } else {
-                        hmid = grow < M ? f4_mul(acc, cur[k]) : f4_zero();
-                    }
-                    st_async4(ring_remote + c * STG_BYTES + row * 128 + ((c8 ^ (row & 7)) << 4), hmid, full_remote);
-                } else if (grow < M) {
+                if (grow < M) {
                     if (OUT == OUT_ADD) acc = f4_add(acc, cur[k]);
                     else acc = f4_add(acc, bv);
                     st4(a.Y + (size_t)grow * 128 + col, acc);
@@ -191,13 +171,14 @@ __device__ __forceinline__ void epilogue_role(const nn_gemm_chain_args& a, const
     }
 }
 
-// Rank-0 epilogue for the tile-transposed layout of the activation-derivative tensor (a.aux_tiled): everything happens in
-// the row-owner layout tcgen05.ld delivers - lane = row.  silu'(q) is written (MID_SILU_SAVE) or read (MID_MUL) as 512
-// contiguous bytes per warp instruction (NN_TILED_INDEX), and the tile for rank 1 is sent from the same registers, so this
-// rank needs NO shared-memory transpose at all (the two-pass staging of the row-major variant was half of the LSU
-// shared-memory traffic of the rank that limits the pair, profiles/r1c_chain_summary.txt).
+// ===================== rank-0 epilogue: mid step -> the peer's ring =====================
+// Everything happens in the row-owner layout tcgen05.ld delivers - lane = row.  The activation-derivative tensor silu'(q) is
+// held tile-transposed (NN_TILED_INDEX): it is written (MID_SILU_SAVE) or read (MID_MUL) as 512 contiguous bytes per warp
+// instruction, and the tile for rank 1 is sent from the same registers, so this rank needs NO shared-memory transpose at
+// all (the two-pass staging of a row-major silu' was half of the LSU shared-memory traffic of the rank that limits the
+// pair, profiles/r1c_chain_summary.txt).
 template <int MID>
-__device__ __forceinline__ void epilogue_rank0_tiled(const nn_gemm_chain_args& a, const ChainCtx& x) {
+__device__ __forceinline__ void epilogue_rank0(const nn_gemm_chain_args& a, const ChainCtx& x) {
     const uint32_t sPst = x.sPst, tmem_base = x.tmem_base;
     const uint32_t bar_t_full = x.bar_t_full, bar_t_empty = x.bar_t_empty, bar_ring_full = x.bar_ring_full,
                    bar_ring_empty = x.bar_ring_empty;
@@ -258,7 +239,7 @@ __device__ __forceinline__ void epilogue_rank0_tiled(const nn_gemm_chain_args& a
                 } else {
                     hmid = live ? f4_mul(acc, cur[j]) : f4_zero();
                 }
-                // ring block of the tiled variant is chunk-major ([chunk j][row]): 512 contiguous bytes per warp instruction on
+                // the ring block is chunk-major ([chunk j][row]): 512 contiguous bytes per warp instruction on
                 // both sides (32 separate 16-byte pieces per instruction through the cluster network were measured slower)
                 st_async4(ring_remote + c * STG_BYTES + j * 512 + lane * 16, hmid, full_remote);
             }
@@ -266,7 +247,7 @@ __device__ __forceinline__ void epilogue_rank0_tiled(const nn_gemm_chain_args& a
     }
 }
 
-template <int MID, int OUT, bool TILED>
+template <int MID, int OUT>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) k_gemm128_chain(nn_gemm_chain_args a_in) {
     // dual launch (Y_b != NULL): even clusters run chain A, odd clusters chain B over the same X tiles
     nn_gemm_chain_args a = a_in;
@@ -377,8 +358,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) k_gemm12
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     const int ch = hf * 4 + j;
-                    const float4 x = (TILED && rank == 1) ? *reinterpret_cast<const float4*>(blk + ch * 512 + lane * 16)
-                                                          : *reinterpret_cast<const float4*>(blk + lane * 128 + ((ch ^ (lane & 7)) << 4));
+                    const float4 x = rank == 1 ? *reinterpret_cast<const float4*>(blk + ch * 512 + lane * 16)
+                                       : *reinterpret_cast<const float4*>(blk + lane * 128 + ((ch ^ (lane & 7)) << 4));
                     const float4 hh = make_float4(tf32_hi(x.x), tf32_hi(x.y), tf32_hi(x.z), tf32_hi(x.w));
                     hi[4 * j] = __float_as_uint(hh.x); hi[4 * j + 1] = __float_as_uint(hh.y);
                     hi[4 * j + 2] = __float_as_uint(hh.z); hi[4 * j + 3] = __float_as_uint(hh.w);
@@ -416,31 +397,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) k_gemm12
                 const uint32_t buf = it & 1, acc_phase = (it >> 1) & 1;
                 mbar_wait(bar_t_empty + 8 * buf, acc_phase ^ 1);
                 tc_fence_after();
-                const uint32_t d_tmem = tmem_base + buf * 128;
-                for (int kb = 0; kb < NKB; ++kb) {
-                    mbar_wait(bar_a_full + 8 * kb, it & 1);
-                    tc_fence_after();
-                    const uint32_t a_hi = tmem_base + A_COL0 + kb * 64, a_lo = a_hi + 32;
-                    const uint32_t b_hi = sB + kb * BLK_BYTES, b_lo = b_hi + NKB * BLK_BYTES;
-#pragma unroll
-                    for (int ks = 0; ks < KB / 8; ++ks) {
-                        const uint64_t dbh = make_desc(b_hi + ks * 32), dbl = make_desc(b_lo + ks * 32);
-                        umma_tf32_ts(d_tmem, a_lo + ks * 8, dbh, (kb | ks) != 0);
-                        umma_tf32_ts(d_tmem, a_hi + ks * 8, dbl, 1);
-                        umma_tf32_ts(d_tmem, a_hi + ks * 8, dbh, 1);
-                    }
-                    umma_commit(bar_a_empty + 8 * kb);
-                }
+                umma_tile_ts(tmem_base + buf * 128, tmem_base + A_COL0, sB, bar_a_full, bar_a_empty, it & 1);
                 umma_commit(bar_t_full + 8 * buf);
             }
         }
         __syncwarp();
     } else {
         asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_EPI));
-        if (rank == 0) {
-            if (TILED) epilogue_rank0_tiled<MID>(a, ctx);
-            else epilogue_role<MID, OUT, 0>(a, ctx);
-        } else epilogue_role<MID, OUT, 1>(a, ctx);
+        if (rank == 0) epilogue_rank0<MID>(a, ctx);
+        else epilogue_rank1<OUT>(a, ctx);
     }
     tc_fence_before();
     cluster_sync_all();                               // no CTA leaves while its peer may still touch its shared memory
@@ -450,29 +415,24 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) k_gemm12
     }
 }
 
-int g_pairs = 0;
-bool g_attr_set[2][2][2] = {};
+bool g_attr_set[2][2] = {};
 
-template <int MID, int OUT, bool TILED>
+template <int MID, int OUT>
 int launch(const nn_gemm_chain_args& a, cudaStream_t s) {
-    if (!g_attr_set[MID][OUT][TILED]) {
-        cudaError_t e = cudaFuncSetAttribute(k_gemm128_chain<MID, OUT, TILED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
+    if (!g_attr_set[MID][OUT]) {
+        cudaError_t e = cudaFuncSetAttribute(k_gemm128_chain<MID, OUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
         if (e != cudaSuccess) { nn_set_error("nn_gemm128_chain: cannot set %u B dynamic smem: %s", SMEM_BYTES, cudaGetErrorString(e)); return -2; }
-        g_attr_set[MID][OUT][TILED] = true;
+        g_attr_set[MID][OUT] = true;
     }
-    if (g_pairs == 0) {
-        int dev = 0, sms = 0; cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        g_pairs = sms > 1 ? sms / 2 : 74;
-    }
+    const int pairs = nn_num_sms() / 2;             // one cluster per pair of SMs
     const int tiles = nn_ceil_div(a.m, TM);
-    int clusters = tiles < g_pairs ? tiles : g_pairs;
+    int clusters = tiles < pairs ? tiles : pairs;
     if (a.Y_b) {                                   // dual: an even number of clusters, half per chain
-        clusters = 2 * tiles < g_pairs ? 2 * tiles : (g_pairs & ~1);
+        clusters = 2 * tiles < pairs ? 2 * tiles : (pairs & ~1);
         if (clusters < 2) clusters = 2;
     }
     NN_LAUNCHED(1);
-    return launch_pdl(k_gemm128_chain<MID, OUT, TILED>, 2 * clusters, THREADS, SMEM_BYTES, s, a);
+    return launch_pdl(k_gemm128_chain<MID, OUT>, 2 * clusters, THREADS, SMEM_BYTES, s, a);
 }
 
 }  // namespace
@@ -489,13 +449,8 @@ extern "C" NN_API int nn_gemm128_chain(const nn_gemm_chain_args* a, void* stream
     if (a->m <= 0) return 0;
     cudaStream_t s = (cudaStream_t)stream;
     int rc;
-    if (a->aux_tiled) {
-        if (a->mid == MID_SILU_SAVE) rc = a->out == OUT_BIAS ? launch<MID_SILU_SAVE, OUT_BIAS, true>(*a, s) : launch<MID_SILU_SAVE, OUT_ADD, true>(*a, s);
-        else rc = a->out == OUT_BIAS ? launch<MID_MUL, OUT_BIAS, true>(*a, s) : launch<MID_MUL, OUT_ADD, true>(*a, s);
-    } else {
-        if (a->mid == MID_SILU_SAVE) rc = a->out == OUT_BIAS ? launch<MID_SILU_SAVE, OUT_BIAS, false>(*a, s) : launch<MID_SILU_SAVE, OUT_ADD, false>(*a, s);
-        else rc = a->out == OUT_BIAS ? launch<MID_MUL, OUT_BIAS, false>(*a, s) : launch<MID_MUL, OUT_ADD, false>(*a, s);
-    }
+    if (a->mid == MID_SILU_SAVE) rc = a->out == OUT_BIAS ? launch<MID_SILU_SAVE, OUT_BIAS>(*a, s) : launch<MID_SILU_SAVE, OUT_ADD>(*a, s);
+    else rc = a->out == OUT_BIAS ? launch<MID_MUL, OUT_BIAS>(*a, s) : launch<MID_MUL, OUT_ADD>(*a, s);
     if (rc) return rc;
     NN_CHECK_LAUNCH("nn_gemm128_chain");
     return 0;

@@ -24,7 +24,6 @@
 namespace {
 
 using namespace tc;
-constexpr int NKB = 4;                        // K blocks per tile (K = 128)
 constexpr int STAGES = 2;
 constexpr uint32_t B_BYTES = 2 * NKB * BLK_BYTES;     // hi + lo image of B = 128 KB
 constexpr uint32_t A_STAGE_BYTES = 2 * BLK_BYTES;     // A_hi + A_lo block = 32 KB
@@ -35,47 +34,6 @@ constexpr int MMA_WARP = PRODUCER_WARPS + EPI_WARPS;
 constexpr int PF = 4;                         // producer register prefetch depth in K blocks (one whole tile)
 constexpr int THREADS = 32 * (PRODUCER_WARPS + EPI_WARPS + 1);
 constexpr uint32_t TMEM_COLS = 256;           // two 128-column fp32 accumulators
-
-// Loads are issued raw (so they stay in flight); the prologue is applied when the value is consumed.
-template <int PRO>
-__device__ __forceinline__ float4 load_a(const nn_gemm_args& a, int grow, int k, int M) {
-    if (grow >= M) return f4_zero();
-    float4 v = ld4(a.X + (size_t)grow * 128 + k);
-    if (PRO == NN_PRO_ROWSCALE3) v = f4_mul(v, ld4(a.aux2 + (size_t)(grow / 3) * 128 + k));
-    return v;
-}
-template <int PRO>
-__device__ __forceinline__ float4 apply_prologue(const nn_gemm_args& a, float4 v, int grow, int k, int M) {
-    if (PRO == NN_PRO_SILU) { v.x = silu_f(v.x); v.y = silu_f(v.y); v.z = silu_f(v.z); v.w = silu_f(v.w); }
-    if (PRO == NN_PRO_SILU_SAVE) {
-        // one sigmoid per element serves silu (this product) and silu' (kept for the reverse sweep)
-        const float4 s = make_float4(sigmoid_f(v.x), sigmoid_f(v.y), sigmoid_f(v.z), sigmoid_f(v.w));
-        if (grow < M)
-            st4(a.aux_out + (size_t)grow * 128 + k,
-                make_float4(s.x * fmaf(v.x, 1.0f - s.x, 1.0f), s.y * fmaf(v.y, 1.0f - s.y, 1.0f),
-                            s.z * fmaf(v.z, 1.0f - s.z, 1.0f), s.w * fmaf(v.w, 1.0f - s.w, 1.0f)));
-        v = f4_mul(v, s);
-    }
-    return v;
-}
-
-template <int EPI>
-__device__ __forceinline__ float4 epilogue(const nn_gemm_args& a, float4 acc, int grow, int col) {
-    if (EPI == NN_EPI_BIAS) {
-        if (a.bias) acc = f4_add(acc, ld4(a.bias + col));
-    } else if (EPI == NN_EPI_DSILU) {
-        float4 p = ld4(a.aux1 + (size_t)grow * 128 + col);
-        acc.x *= dsilu_f(p.x); acc.y *= dsilu_f(p.y); acc.z *= dsilu_f(p.z); acc.w *= dsilu_f(p.w);
-    } else if (EPI == NN_EPI_ADD) {
-        acc = f4_add(acc, ld4(a.aux1 + (size_t)grow * 128 + col));
-    } else if (EPI == NN_EPI_EQUIV_BWD) {
-        float4 fb = ld4(a.aux1 + (size_t)grow * 128 + col);
-        float4 ab = ld4(a.aux2 + (size_t)(grow / 3) * 128 + col);
-        float4 g = ld4(a.aux3 + (size_t)grow * 128 + col);
-        acc = f4_add(acc, f4_fma(ab, g, fb));
-    }
-    return acc;
-}
 
 template <int PRO, int EPI>
 __global__ void __launch_bounds__(THREADS, 1) k_gemm128_tc(nn_gemm_args a) {
@@ -303,7 +261,6 @@ __global__ void k_prepare_b_batch(PrepBatch p) {
     img[(NKB * BLK_BYTES + off) / 4] = x - hi;
 }
 
-int g_num_sms = 0;
 bool g_attr_set[4][5] = {};
 
 template <int PRO, int EPI>
@@ -313,13 +270,8 @@ int launch(const nn_gemm_args& a, cudaStream_t s) {
         if (e != cudaSuccess) { nn_set_error("nn_gemm128(tc): cannot set %u B dynamic smem: %s", SMEM_BYTES, cudaGetErrorString(e)); return -2; }
         g_attr_set[PRO][EPI] = true;
     }
-    if (g_num_sms == 0) {
-        int dev = 0; cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
-        if (g_num_sms <= 0) g_num_sms = 148;
-    }
-    int tiles = nn_ceil_div(a.m, TM);
-    int grid = tiles < g_num_sms ? tiles : g_num_sms;
+    const int tiles = nn_ceil_div(a.m, TM), sms = nn_num_sms();
+    const int grid = tiles < sms ? tiles : sms;
     k_gemm128_tc<PRO, EPI><<<grid, THREADS, SMEM_BYTES, s>>>(a); NN_LAUNCHED(1);
     return 0;
 }

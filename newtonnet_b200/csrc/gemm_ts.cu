@@ -18,7 +18,6 @@
 namespace {
 
 using namespace tc;
-constexpr int NKB = 4;                        // K blocks per tile (K = 128)
 constexpr uint32_t B_BYTES = 2 * NKB * BLK_BYTES;     // hi + lo image of B = 128 KB
 constexpr uint32_t BAR_BYTES = 256;
 constexpr int PDEPTH = 2;                     // cp.async staging buffers per producer warp (items in flight)
@@ -38,55 +37,9 @@ static_assert(256 * REGS_PROD + 256 * REGS_EPI + 128 * REGS_MMA <= 640 * 96, "re
 constexpr uint32_t TMEM_COLS = 512;           // 2 x 128 accumulator columns + 4 K blocks x 64 columns of A
 constexpr uint32_t A_COL0 = 256;
 
-// Loads are issued raw (so they stay in flight); the prologue is applied when the value is consumed.
-template <int PRO>
-__device__ __forceinline__ float4 load_a(const nn_gemm_args& a, int grow, int k, int M) {
-    if (grow >= M) return f4_zero();
-    float4 v = ld4(a.X + (size_t)grow * 128 + k);
-    if (PRO == NN_PRO_ROWSCALE3) v = f4_mul(v, ld4(a.aux2 + (size_t)(grow / 3) * 128 + k));
-    return v;
-}
-template <int PRO>
-__device__ __forceinline__ float4 apply_prologue(const nn_gemm_args& a, float4 v, int grow, int k, int M) {
-    if (PRO == NN_PRO_SILU) { v.x = silu_f(v.x); v.y = silu_f(v.y); v.z = silu_f(v.z); v.w = silu_f(v.w); }
-    if (PRO == NN_PRO_SILU_SAVE) {
-        // one sigmoid per element serves silu (this product) and silu' (kept for the reverse sweep)
-        const float4 s = make_float4(sigmoid_f(v.x), sigmoid_f(v.y), sigmoid_f(v.z), sigmoid_f(v.w));
-        if (grow < M)
-            st4(a.aux_out + (size_t)grow * 128 + k,
-                make_float4(s.x * fmaf(v.x, 1.0f - s.x, 1.0f), s.y * fmaf(v.y, 1.0f - s.y, 1.0f),
-                            s.z * fmaf(v.z, 1.0f - s.z, 1.0f), s.w * fmaf(v.w, 1.0f - s.w, 1.0f)));
-        v = f4_mul(v, s);
-    }
-    return v;
-}
-
-template <int EPI>
-__device__ __forceinline__ float4 epilogue(const nn_gemm_args& a, float4 acc, int grow, int col) {
-    if (EPI == NN_EPI_BIAS) {
-        if (a.bias) acc = f4_add(acc, ld4(a.bias + col));
-    } else if (EPI == NN_EPI_DSILU) {
-        float4 p = ld4(a.aux1 + (size_t)grow * 128 + col);
-        acc.x *= dsilu_f(p.x); acc.y *= dsilu_f(p.y); acc.z *= dsilu_f(p.z); acc.w *= dsilu_f(p.w);
-    } else if (EPI == NN_EPI_ADD) {
-        acc = f4_add(acc, ld4(a.aux1 + (size_t)grow * 128 + col));
-    } else if (EPI == NN_EPI_EQUIV_BWD) {
-        float4 fb = ld4(a.aux1 + (size_t)grow * 128 + col);
-        float4 ab = ld4(a.aux2 + (size_t)(grow / 3) * 128 + col);
-        float4 g = ld4(a.aux3 + (size_t)grow * 128 + col);
-        acc = f4_add(acc, f4_fma(ab, g, fb));
-    }
-    return acc;
-}
-
-// TILED: the EPI_MUL factor aux1 is tile-transposed; XT / YT: X / Y are tile-transposed (NN_TILED_INDEX) - a producer then
-// loads its rows straight into registers (no cp.async staging, no shared-memory read) and an epilogue stores straight from
-// the tcgen05.ld registers (no staging transpose): the intermediate of a two-launch reverse MLP travels in that layout.
-template <int PRO, int EPI, bool TILED = false, bool XT = false, bool YT = false>
+// TILED: the EPI_MUL factor aux1 is tile-transposed (NN_TILED_INDEX), as the chained kernel writes it
+template <int PRO, int EPI, bool TILED = false>
 __global__ void __launch_bounds__(THREADS, 1) k_gemm128_ts(nn_gemm_args a) {
-    // register split per variant: a producer that holds its rows in registers needs more, its plain epilogue less
-    constexpr int kRegsProd = XT ? 120 : REGS_PROD, kRegsEpi = XT ? 88 : REGS_EPI;
-    static_assert(256 * kRegsProd + 256 * kRegsEpi + 128 * REGS_MMA <= 640 * 96, "register budget");
     extern __shared__ uint8_t smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;          // swizzle atoms need 1024 B alignment
     const uint32_t sB = base;                                             // [hi|lo][kb][16 KB]
@@ -130,54 +83,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_gemm128_ts(nn_gemm_args a) {
     const int n_tiles = (M + TM - 1) / TM;
     const bool has_work = (int)blockIdx.x < n_tiles;
 
-    if (XT && warp < PRODUCER_WARPS) {
-        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kRegsProd));
-        // ===================== producers, tile-transposed X: rows -> registers -> hi/lo split -> TMEM =====================
-        const int q = warp & 3, h = warp >> 2;
-        const int rt = q * 32 + lane;
-        const int my_tiles = has_work ? (n_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
-        const int n_items = my_tiles * 2;                 // item w = (tile w >> 1, K block 2h + (w & 1))
-        float4 cur[8], nxt[8];
-        auto load = [&](int w, float4 (&dst)[8]) {
-            const int tile = (int)blockIdx.x + (w >> 1) * (int)gridDim.x, kb = 2 * h + (w & 1);
-            const bool ok = w < n_items && tile * TM + rt < M;      // rows beyond M read as zeros
-#pragma unroll
-            for (int ch = 0; ch < 8; ++ch)
-                dst[ch] = ok ? ld4(a.X + (((size_t)tile * 32 + kb * 8 + ch) * 128 + rt) * 4) : f4_zero();
-        };
-        load(0, cur);
-        for (int w = 0; w < n_items; ++w) {
-            const int t_local = w >> 1, kb = 2 * h + (w & 1);
-            load(w + 1, nxt);                                 // the next item's rows are in flight while this one is split
-            const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + A_COL0 + kb * 64;
-            bool waited = false;
-#pragma unroll
-            for (int hf = 0; hf < 2; ++hf) {
-                uint32_t hi[16], lo[16];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const float4 x = cur[hf * 4 + j];
-                    const float4 hh = make_float4(tf32_hi(x.x), tf32_hi(x.y), tf32_hi(x.z), tf32_hi(x.w));
-                    hi[4 * j] = __float_as_uint(hh.x); hi[4 * j + 1] = __float_as_uint(hh.y);
-                    hi[4 * j + 2] = __float_as_uint(hh.z); hi[4 * j + 3] = __float_as_uint(hh.w);
-                    lo[4 * j] = __float_as_uint(x.x - hh.x); lo[4 * j + 1] = __float_as_uint(x.y - hh.y);
-                    lo[4 * j + 2] = __float_as_uint(x.z - hh.z); lo[4 * j + 3] = __float_as_uint(x.w - hh.w);
-                }
-                if (!waited) {
-                    mbar_wait(bar_a_empty + 8 * kb, (t_local & 1) ^ 1);
-                    tc_fence_after();
-                    waited = true;
-                }
-                tmem_st16(taddr + hf * 16, hi);
-                tmem_st16(taddr + 32 + hf * 16, lo);
-            }
-            tmem_st_wait();
-            tc_fence_before();
-            mbar_arrive(bar_a_full + 8 * kb);
-#pragma unroll
-            for (int ch = 0; ch < 8; ++ch) cur[ch] = nxt[ch];
-        }
-    } else if (warp < PRODUCER_WARPS) {
+    if (warp < PRODUCER_WARPS) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_PROD));
         // ===================== producers: X rows -> transpose -> hi/lo split -> TMEM =====================
         // warp = (lane quarter q, K-block half h): rows [32q, 32q+32) of K blocks 2h and 2h+1 of every tile.
@@ -257,28 +163,13 @@ __global__ void __launch_bounds__(THREADS, 1) k_gemm128_ts(nn_gemm_args a) {
                 const uint32_t buf = it & 1, acc_phase = (it >> 1) & 1;
                 mbar_wait(bar_t_empty + 8 * buf, acc_phase ^ 1);          // epilogue has drained this accumulator
                 tc_fence_after();
-                const uint32_t d_tmem = tmem_base + buf * 128;
-                for (int kb = 0; kb < NKB; ++kb) {
-                    mbar_wait(bar_a_full + 8 * kb, it & 1);
-                    tc_fence_after();
-                    const uint32_t a_hi = tmem_base + A_COL0 + kb * 64, a_lo = a_hi + 32;
-                    const uint32_t b_hi = sB + kb * BLK_BYTES, b_lo = b_hi + NKB * BLK_BYTES;
-#pragma unroll
-                    for (int ks = 0; ks < KB / 8; ++ks) {                  // UMMA_K = 8 tf32 = 8 TMEM columns / 32 bytes
-                        const uint64_t dbh = make_desc(b_hi + ks * 32), dbl = make_desc(b_lo + ks * 32);
-                        umma_tf32_ts(d_tmem, a_lo + ks * 8, dbh, (kb | ks) != 0);   // small terms first
-                        umma_tf32_ts(d_tmem, a_hi + ks * 8, dbl, 1);
-                        umma_tf32_ts(d_tmem, a_hi + ks * 8, dbh, 1);
-                    }
-                    umma_commit(bar_a_empty + 8 * kb);                     // K block's TMEM columns reusable
-                }
+                umma_tile_ts(tmem_base + buf * 128, tmem_base + A_COL0, sB, bar_a_full, bar_a_empty, it & 1);
                 umma_commit(bar_t_full + 8 * buf);                         // accumulator complete
             }
         }
         __syncwarp();
     } else {
-        if (XT) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kRegsEpi));
-        else asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kRegsEpi));
+        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_EPI));
         // ===================== epilogue: TMEM -> registers -> smem transpose -> global =====================
         // 8 warps: TMEM lane quarter q = warp % 4 (hardware restriction), column half = (warp - 8) / 4.
         // tcgen05.ld hands every lane one accumulator ROW; storing that straight to global memory would
@@ -294,11 +185,10 @@ __global__ void __launch_bounds__(THREADS, 1) k_gemm128_ts(nn_gemm_args a) {
         float4 ax[8];
         // EPI_MUL with a tile-transposed factor (a.aux_tiled, written by the chained kernel): the factor is read and applied
         // in the row-owner layout, straight after tcgen05.ld (lane = row: 512 contiguous bytes per warp instruction)
-        constexpr bool tiled = TILED;
         const int rt = q * 32 + lane;
         auto prefetch = [&](int tile, int c0) {
             if (!kAux1) return;
-            if (tiled) {
+            if (TILED) {
 #pragma unroll
                 for (int j = 0; j < 8; ++j) ax[j] = ld4(a.aux1 + (((size_t)tile * 32 + (c0 >> 2) + j) * 128 + rt) * 4);
                 return;
@@ -325,7 +215,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_gemm128_ts(nn_gemm_args a) {
                     tc_fence_before();
                     mbar_arrive(bar_t_empty + 8 * buf);
                 }
-                if (tiled) {
+                if (TILED) {
 #pragma unroll
                     for (int j = 0; j < 8; ++j) {
                         v[4 * j] = __float_as_uint(__uint_as_float(v[4 * j]) * ax[j].x);
@@ -336,19 +226,6 @@ __global__ void __launch_bounds__(THREADS, 1) k_gemm128_ts(nn_gemm_args a) {
                     if (c == 0) prefetch(tile, c0 + 32);
                     else if (tile + (int)gridDim.x < n_tiles) prefetch(tile + gridDim.x, half * 64);
                 }
-                if (YT) {                            // tile-transposed output: 512 contiguous bytes per warp instruction, no staging
-                    static_assert(!YT || (EPI == NN_EPI_MUL && TILED) || EPI == NN_EPI_BIAS, "tiled output: MUL (tiled factor) or plain");
-                    if (tile * TM + rt < M) {
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) {
-                            float4 o = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
-                                                   __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-                            if (EPI == NN_EPI_BIAS && a.bias) o = f4_add(o, ld4(a.bias + c0 + 4 * j));
-                            st4(a.Y + (((size_t)tile * 32 + (c0 >> 2) + j) * 128 + rt) * 4, o);
-                        }
-                    }
-                    continue;
-                }
 #pragma unroll
                 for (int j = 0; j < 8; ++j)         // row = lane, 16-byte chunk j -> physical chunk j ^ (lane & 7)
                     *reinterpret_cast<float4*>(stg + lane * 128 + ((j ^ (lane & 7)) << 4)) =
@@ -356,7 +233,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_gemm128_ts(nn_gemm_args a) {
                                     __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
                 __syncwarp();
                 float4 cur[8];
-                if (kAux1 && !tiled) {
+                if (kAux1 && !TILED) {
 #pragma unroll
                     for (int k = 0; k < 8; ++k) cur[k] = ax[k];
                     if (c == 0) prefetch(tile, c0 + 32);
@@ -375,7 +252,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_gemm128_ts(nn_gemm_args a) {
                         } else if (EPI == NN_EPI_ADD) {
                             acc = f4_add(acc, cur[k]);
                         } else if (EPI == NN_EPI_MUL) {
-                            if (!tiled) acc = f4_mul(acc, cur[k]);
+                            if (!TILED) acc = f4_mul(acc, cur[k]);
                         } else {
                             acc = epilogue<EPI>(a, acc, grow, col);
                         }
@@ -394,25 +271,19 @@ __global__ void __launch_bounds__(THREADS, 1) k_gemm128_ts(nn_gemm_args a) {
     }
 }
 
-int g_num_sms = 0;
-bool g_attr_set[4][5][2][2][2] = {};
+bool g_attr_set[4][5][2] = {};
 
-template <int PRO, int EPI, bool TILED = false, bool XT = false, bool YT = false>
+template <int PRO, int EPI, bool TILED = false>
 int launch(const nn_gemm_args& a, cudaStream_t s) {
-    if (!g_attr_set[PRO][EPI][TILED][XT][YT]) {
-        cudaError_t e = cudaFuncSetAttribute(k_gemm128_ts<PRO, EPI, TILED, XT, YT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
+    if (!g_attr_set[PRO][EPI][TILED]) {
+        cudaError_t e = cudaFuncSetAttribute(k_gemm128_ts<PRO, EPI, TILED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
         if (e != cudaSuccess) { nn_set_error("nn_gemm128(ts): cannot set %u B dynamic smem: %s", SMEM_BYTES, cudaGetErrorString(e)); return -2; }
-        g_attr_set[PRO][EPI][TILED][XT][YT] = true;
+        g_attr_set[PRO][EPI][TILED] = true;
     }
-    if (g_num_sms == 0) {
-        int dev = 0; cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
-        if (g_num_sms <= 0) g_num_sms = 148;
-    }
-    int tiles = nn_ceil_div(a.m, TM);
-    int grid = tiles < g_num_sms ? tiles : g_num_sms;
+    const int tiles = nn_ceil_div(a.m, TM), sms = nn_num_sms();
+    const int grid = tiles < sms ? tiles : sms;
     NN_LAUNCHED(1);
-    return launch_pdl(k_gemm128_ts<PRO, EPI, TILED, XT, YT>, grid, THREADS, SMEM_BYTES, s, a);
+    return launch_pdl(k_gemm128_ts<PRO, EPI, TILED>, grid, THREADS, SMEM_BYTES, s, a);
 }
 
 }  // namespace
@@ -422,14 +293,6 @@ int nn_gemm128_ts_launch(const nn_gemm_args& a, cudaStream_t s) {
     NN_REQUIRE(a.B_img != nullptr, "tensor-core backend needs B_img (nn_gemm128_prepare_b)");
     int rc = -1;
 #define NN_CASE(P, E) if (a.prologue == P && a.epilogue == E) { rc = launch<P, E>(a, s); goto done; }
-    if (a.xy_tiled) {
-        // tile-transposed X (bit 0) / Y (bit 1): the two launches of a reverse MLP handing their intermediate over in that layout
-        if (a.prologue == NN_PRO_NONE && a.epilogue == NN_EPI_MUL && a.aux_tiled && a.xy_tiled == 2) { rc = launch<NN_PRO_NONE, NN_EPI_MUL, true, false, true>(a, s); goto done; }
-        if (a.prologue == NN_PRO_NONE && a.epilogue == NN_EPI_BIAS && a.xy_tiled == 1) { rc = launch<NN_PRO_NONE, NN_EPI_BIAS, false, true, false>(a, s); goto done; }
-        nn_set_error("nn_gemm128: unsupported tile-transposed combination (prologue %d, epilogue %d, aux_tiled %d, xy_tiled %d)",
-                     a.prologue, a.epilogue, a.aux_tiled, a.xy_tiled);
-        return -1;
-    }
     NN_CASE(NN_PRO_NONE, NN_EPI_BIAS)
     NN_CASE(NN_PRO_SILU, NN_EPI_BIAS)
     NN_CASE(NN_PRO_NONE, NN_EPI_DSILU)

@@ -334,7 +334,6 @@ __global__ void k_message_prepare_b(const float* __restrict__ We, float* __restr
     img[(BLK_BYTES + off) / 4] = x - hi;
 }
 
-int g_sms = 0;
 bool g_attr[2] = {false, false};
 
 template <bool BWD>
@@ -345,13 +344,8 @@ int launch(const MsgArgs& a, cudaStream_t s) {
         if (e != cudaSuccess) { nn_set_error("message_tc: cannot set %u B dynamic smem: %s", C::SMEM, cudaGetErrorString(e)); return -2; }
         g_attr[BWD] = true;
     }
-    if (g_sms == 0) {
-        int dev = 0; cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&g_sms, cudaDevAttrMultiProcessorCount, dev);
-        if (g_sms <= 0) g_sms = 148;
-    }
-    int tiles = nn_ceil_div(a.cap, TM);
-    int grid = tiles < g_sms ? tiles : g_sms;
+    const int tiles = nn_ceil_div(a.cap, TM), sms = nn_num_sms();
+    const int grid = tiles < sms ? tiles : sms;
     NN_LAUNCHED(1);
     return launch_pdl(k_message_tc<BWD>, grid, THREADS, C::SMEM, s, a);
 }

@@ -52,7 +52,6 @@ k_edge_geom_fwd(const float* __restrict__ disp, const float* __restrict__ freq, 
                 const int* __restrict__ n_dev, int cap, float* __restrict__ rbf,
                 float* __restrict__ drbf, float* __restrict__ unit, float* __restrict__ dist) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     static_assert(kNB == 20, "five float4 per basis row");
     const int P = dev_count(n_dev, cap);
     const long long total = (long long)P * 5;
@@ -88,7 +87,6 @@ __global__ void k_edge_geom_bwd(const float* __restrict__ x_bar, int n_slots, co
                                 const float* __restrict__ unit, const float* __restrict__ dist, float cutoff,
                                 const int* __restrict__ n_dev, int cap, float* __restrict__ disp_bar) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     const int P = dev_count(n_dev, cap);
     for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < P; p += gridDim.x * blockDim.x) {
         float d = dist[p];
@@ -167,7 +165,6 @@ k_node_aggregate_fwd(const int* __restrict__ status, const int* __restrict__ row
                      const float* __restrict__ e2, const float* __restrict__ unit, const float* __restrict__ a_in,
                      const float* __restrict__ f_in, float* __restrict__ a_out, float* __restrict__ f_out) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     const int lane = threadIdx.x & 31;
     const int i = blockIdx.x * kAggWarps + (threadIdx.x >> 5);
     if (i >= N || status[NN_ST_EDGE_OVERFLOW] != 0) return;   // overflow: row_ptr is ahead of col / edge_pair
@@ -215,7 +212,6 @@ k_node_aggregate_fwd(const int* __restrict__ status, const int* __restrict__ row
 __global__ void k_equiv_update_fwd(const float* __restrict__ a_in, const float* __restrict__ f,
                                    const float* __restrict__ g, float* __restrict__ a_out, int N) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     int t = blockIdx.x * blockDim.x + threadIdx.x;       // one float4 of one atom
     if (t >= N * (kF / 4)) return;
     int i = t / (kF / 4), q = (t % (kF / 4)) * 4;
@@ -231,7 +227,6 @@ __global__ void k_equiv_update_fwd(const float* __restrict__ a_in, const float* 
 __global__ void k_embed(const int64_t* __restrict__ z, const float* __restrict__ emb, float* __restrict__ a, int N,
                         int* __restrict__ status) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= N * (kF / 4)) return;
     int i = t / (kF / 4), q = (t % (kF / 4)) * 4;
@@ -246,7 +241,6 @@ __global__ void __launch_bounds__(kThreads)
 k_layer_norm_fwd(float* __restrict__ a_io, const float* __restrict__ gamma, const float* __restrict__ beta,
                  float* __restrict__ xhat, float* __restrict__ rstd, int n_rows) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     const int lane = threadIdx.x & 31;
     const int i = blockIdx.x * kWarps + (threadIdx.x >> 5);
     if (i >= n_rows) return;
@@ -265,7 +259,6 @@ __global__ void __launch_bounds__(kThreads)
 k_layer_norm_bwd(float* __restrict__ abar_io, const float* __restrict__ gamma, const float* __restrict__ xhat,
                  const float* __restrict__ rstd, int n_rows) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     const int lane = threadIdx.x & 31;
     const int i = blockIdx.x * kWarps + (threadIdx.x >> 5);
     if (i >= n_rows) return;
@@ -301,7 +294,6 @@ k_energy_atom(const float* __restrict__ h2pre, const float* __restrict__ w3, con
               const float* __restrict__ scale, const float* __restrict__ shift, const int64_t* __restrict__ z,
               int N, float* __restrict__ e_atom) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     const int lane = threadIdx.x & 31;
     const int i = blockIdx.x * kWarps + (threadIdx.x >> 5);
     if (i >= N) return;
@@ -371,7 +363,6 @@ __global__ void k_energy_head_seed(const float* __restrict__ h2pre, const float*
                                    const float* __restrict__ scale, const int64_t* __restrict__ z, int N,
                                    float* __restrict__ gh2) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= N * (kF / 4)) return;
     int i = t / (kF / 4), q = (t % (kF / 4)) * 4;
@@ -395,7 +386,6 @@ k_pair_bwd_gather(const int* __restrict__ pair_ptr, const int* __restrict__ pair
                   const float* __restrict__ unit, float* __restrict__ e1_io, float* __restrict__ e2bar,
                   float* __restrict__ ubar) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     const int lane = threadIdx.x & 31;
     for (int i = blockIdx.x * kWarps + (threadIdx.x >> 5); i < N; i += gridDim.x * kWarps) {
         const int p0 = pair_ptr[i], p1 = min(pair_ptr[i + 1], cap);
@@ -515,7 +505,6 @@ k_node_aggregate_bwd(const int* __restrict__ status, const int* __restrict__ row
                      const int* __restrict__ edge_pair, int N, const float* __restrict__ t, const float* __restrict__ mn, const float* __restrict__ e2,
                      const float* __restrict__ dfb, float* __restrict__ mnbar, float* __restrict__ fbar_new) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     const int lane = threadIdx.x & 31;
     const int k = blockIdx.x * kAggWarps + (threadIdx.x >> 5);
     if (k >= N || status[NN_ST_EDGE_OVERFLOW] != 0) return;
@@ -562,7 +551,6 @@ k_force_virial_atom(const int* __restrict__ status, const int* __restrict__ row_
                     const int64_t* __restrict__ batch, const SysMeta* __restrict__ meta,
                     float* __restrict__ forces, float* __restrict__ vir_atom) {
     NN_PDL_TRIGGER();
-    NN_PDL_WAIT();
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_rows || status[NN_ST_EDGE_OVERFLOW] != 0) return;
     const int r0 = row_ptr[i], r1 = row_ptr[i + 1];
@@ -704,7 +692,7 @@ extern "C" int nn_edge_geom_fwd(const float* pair_disp, const float* freq, float
                                 int32_t cap_pairs, float* rbf, float* drbf, float* unit, float* dist, void* stream) {
     if (cap_pairs <= 0) return 0;
     int grid = min(nn_ceil_div((long long)cap_pairs * 5, 320), nn_num_sms() * 6);
-    nn_launch_dep(k_edge_geom_fwd, dim3(grid), dim3(320), 0, (cudaStream_t)stream, pair_disp, freq, cutoff, n_pairs_dev, cap_pairs, rbf, drbf, unit, dist); NN_LAUNCHED(1);
+    k_edge_geom_fwd<<<grid, 320, 0, (cudaStream_t)stream>>>(pair_disp, freq, cutoff, n_pairs_dev, cap_pairs, rbf, drbf, unit, dist); NN_LAUNCHED(1);
     NN_CHECK_LAUNCH("nn_edge_geom_fwd");
     return 0;
 }
@@ -714,8 +702,8 @@ extern "C" int nn_edge_geom_bwd(const float* x_bar, int32_t n_slots, const float
                                 float* disp_bar, void* stream) {
     if (cap_pairs <= 0) return 0;
     int grid = min(nn_ceil_div(cap_pairs, 256), nn_num_sms() * 8);
-    nn_launch_dep(k_edge_geom_bwd, dim3(grid), dim3(256), 0, (cudaStream_t)stream, x_bar, n_slots, unit_bar, unit, dist, cutoff, n_pairs_dev, cap_pairs,
-                                                           disp_bar); NN_LAUNCHED(1);
+    k_edge_geom_bwd<<<grid, 256, 0, (cudaStream_t)stream>>>(x_bar, n_slots, unit_bar, unit, dist, cutoff, n_pairs_dev, cap_pairs,
+                                                            disp_bar); NN_LAUNCHED(1);
     NN_CHECK_LAUNCH("nn_edge_geom_bwd");
     return 0;
 }
@@ -746,12 +734,12 @@ int nn_node_aggregate_fwd_rows(const nn_nbr* nl, int n_rows, const float* msg, c
     if (N <= 0) return 0;
     int grid = nn_ceil_div(N, kAggWarps);
     if (first_layer) {
-        nn_launch_dep(k_node_aggregate_fwd<true>, dim3(grid), dim3(kAggThreads), 0, (cudaStream_t)stream, nl->status, nl->row_ptr, nl->col, nl->edge_pair, N, msg,
-                                                                                e1, e2, unit, a_in, f_in, a_out, f_out); NN_LAUNCHED(1);
+        k_node_aggregate_fwd<true><<<grid, kAggThreads, 0, (cudaStream_t)stream>>>(nl->status, nl->row_ptr, nl->col, nl->edge_pair, N, msg,
+                                                                                   e1, e2, unit, a_in, f_in, a_out, f_out); NN_LAUNCHED(1);
     }
     else {
-        nn_launch_dep(k_node_aggregate_fwd<false>, dim3(grid), dim3(kAggThreads), 0, (cudaStream_t)stream, nl->status, nl->row_ptr, nl->col, nl->edge_pair, N, msg,
-                                                                                 e1, e2, unit, a_in, f_in, a_out, f_out); NN_LAUNCHED(1);
+        k_node_aggregate_fwd<false><<<grid, kAggThreads, 0, (cudaStream_t)stream>>>(nl->status, nl->row_ptr, nl->col, nl->edge_pair, N, msg,
+                                                                                    e1, e2, unit, a_in, f_in, a_out, f_out); NN_LAUNCHED(1);
     }
     NN_CHECK_LAUNCH("nn_node_aggregate_fwd");
     return 0;
@@ -760,7 +748,7 @@ int nn_node_aggregate_fwd_rows(const nn_nbr* nl, int n_rows, const float* msg, c
 extern "C" int nn_equiv_update_fwd(const float* a_in, const float* f, const float* g, float* a_out, int32_t n_atoms,
                                    void* stream) {
     if (n_atoms <= 0) return 0;
-    nn_launch_dep(k_equiv_update_fwd, dim3(nn_ceil_div((long long)n_atoms * (kF / 4), 256)), dim3(256), 0, (cudaStream_t)stream, a_in, f, g, a_out, n_atoms); NN_LAUNCHED(1);
+    k_equiv_update_fwd<<<nn_ceil_div((long long)n_atoms * (kF / 4), 256), 256, 0, (cudaStream_t)stream>>>(a_in, f, g, a_out, n_atoms); NN_LAUNCHED(1);
     NN_CHECK_LAUNCH("nn_equiv_update_fwd");
     return 0;
 }
@@ -784,7 +772,7 @@ int nn_energy_head_fwd_rows(const float* h2pre, const float* w3, const float* b3
                             const int64_t* z, const int32_t* sys_ptr, int n_atoms, int n_systems, float* e_atom,
                             float* energy, double* partial, int slices, cudaStream_t s) {
     if (n_atoms > 0) {
-        nn_launch_dep(k_energy_atom, dim3(nn_ceil_div(n_atoms, kWarps)), dim3(kThreads), 0, s, h2pre, w3, b3, scale, shift, z, n_atoms, e_atom); NN_LAUNCHED(1);
+        k_energy_atom<<<nn_ceil_div(n_atoms, kWarps), kThreads, 0, s>>>(h2pre, w3, b3, scale, shift, z, n_atoms, e_atom); NN_LAUNCHED(1);
     }
     if (partial && slices > 1) {
         k_sys_sum_partial<1><<<dim3(n_systems, slices), kThreads, 0, s>>>(e_atom, sys_ptr, n_atoms, slices, partial); NN_LAUNCHED(1);
@@ -801,9 +789,9 @@ int nn_force_virial_rows(const nn_nbr* nl, int n_rows, const float* disp_bar, fl
     float* vir_atom = virial ? (float*)workspace : nullptr;
     NN_REQUIRE(!virial || workspace, "virial needs a workspace of n_atoms*9 floats");
     if (n_rows > 0) {
-        nn_launch_dep(k_force_virial_atom, dim3(nn_ceil_div(n_rows, 128)), dim3(128), 0, s, nl->status, nl->row_ptr, nl->col, nl->edge_pair, n_rows,
-                                                                      disp_bar, nl->pair_disp, nl->pos, nl->batch,
-                                                                      nn_nbr_sysmeta(nl), forces, vir_atom); NN_LAUNCHED(1);
+        k_force_virial_atom<<<nn_ceil_div(n_rows, 128), 128, 0, s>>>(nl->status, nl->row_ptr, nl->col, nl->edge_pair, n_rows,
+                                                                     disp_bar, nl->pair_disp, nl->pos, nl->batch,
+                                                                     nn_nbr_sysmeta(nl), forces, vir_atom); NN_LAUNCHED(1);
     }
     if (virial && partial && slices > 1) {
         k_sys_sum_partial<9><<<dim3(nl->n_systems, slices), kThreads, 0, s>>>(vir_atom, nl->sys_ptr, n_rows, slices, partial); NN_LAUNCHED(1);
@@ -832,13 +820,13 @@ extern "C" int nn_halo_pack(const float* src, const int32_t* idx, int32_t n, int
 // ---- launchers used only by nn_eval (eval.cu)
 int nn_layer_norm_fwd_launch(float* a_io, const float* gamma, const float* beta, float* xhat, float* rstd, int n_rows, cudaStream_t s) {
     if (n_rows <= 0) return 0;
-    nn_launch_dep(k_layer_norm_fwd, dim3(nn_ceil_div(n_rows, kWarps)), dim3(kThreads), 0, s, a_io, gamma, beta, xhat, rstd, n_rows); NN_LAUNCHED(1);
+    k_layer_norm_fwd<<<nn_ceil_div(n_rows, kWarps), kThreads, 0, s>>>(a_io, gamma, beta, xhat, rstd, n_rows); NN_LAUNCHED(1);
     NN_CHECK_LAUNCH("layer_norm_fwd");
     return 0;
 }
 int nn_layer_norm_bwd_launch(float* abar_io, const float* gamma, const float* xhat, const float* rstd, int n_rows, cudaStream_t s) {
     if (n_rows <= 0) return 0;
-    nn_launch_dep(k_layer_norm_bwd, dim3(nn_ceil_div(n_rows, kWarps)), dim3(kThreads), 0, s, abar_io, gamma, xhat, rstd, n_rows); NN_LAUNCHED(1);
+    k_layer_norm_bwd<<<nn_ceil_div(n_rows, kWarps), kThreads, 0, s>>>(abar_io, gamma, xhat, rstd, n_rows); NN_LAUNCHED(1);
     NN_CHECK_LAUNCH("layer_norm_bwd");
     return 0;
 }
@@ -850,14 +838,14 @@ int nn_direct_force_launch(const float* h, const float* f, const float* scale, c
 }
 int nn_embed_launch(const int64_t* z, const float* emb, float* a, int N, int* status, cudaStream_t s) {
     if (N <= 0) return 0;
-    nn_launch_dep(k_embed, dim3(nn_ceil_div((long long)N * (kF / 4), 256)), dim3(256), 0, s, z, emb, a, N, status); NN_LAUNCHED(1);
+    k_embed<<<nn_ceil_div((long long)N * (kF / 4), 256), 256, 0, s>>>(z, emb, a, N, status); NN_LAUNCHED(1);
     NN_CHECK_LAUNCH("embed");
     return 0;
 }
 int nn_energy_head_seed_launch(const float* h2pre, const float* w3, const float* scale, const int64_t* z, int N,
                                float* gh2, cudaStream_t s) {
     if (N <= 0) return 0;
-    nn_launch_dep(k_energy_head_seed, dim3(nn_ceil_div((long long)N * (kF / 4), 256)), dim3(256), 0, s, h2pre, w3, scale, z, N, gh2); NN_LAUNCHED(1);
+    k_energy_head_seed<<<nn_ceil_div((long long)N * (kF / 4), 256), 256, 0, s>>>(h2pre, w3, scale, z, N, gh2); NN_LAUNCHED(1);
     NN_CHECK_LAUNCH("energy_head_seed");
     return 0;
 }
@@ -866,12 +854,12 @@ int nn_pair_bwd_gather_launch(const nn_nbr* nl, const float* dfb, const float* f
     if (nl->cap_pairs <= 0) return 0;
     int grid = grid_for_rows(nl->n_atoms);
     if (first) {
-        nn_launch_dep(k_pair_bwd_gather<true>, dim3(grid), dim3(kThreads), 0, s, nl->pair_ptr, nl->pair_j, nl->n_atoms, nl->cap_pairs,
-                                                           dfb, f_in, unit, e1_io, e2bar, ubar); NN_LAUNCHED(1);
+        k_pair_bwd_gather<true><<<grid, kThreads, 0, s>>>(nl->pair_ptr, nl->pair_j, nl->n_atoms, nl->cap_pairs,
+                                                          dfb, f_in, unit, e1_io, e2bar, ubar); NN_LAUNCHED(1);
     }
     else {
-        nn_launch_dep(k_pair_bwd_gather<false>, dim3(grid), dim3(kThreads), 0, s, nl->pair_ptr, nl->pair_j, nl->n_atoms, nl->cap_pairs,
-                                                            dfb, f_in, unit, e1_io, e2bar, ubar); NN_LAUNCHED(1);
+        k_pair_bwd_gather<false><<<grid, kThreads, 0, s>>>(nl->pair_ptr, nl->pair_j, nl->n_atoms, nl->cap_pairs,
+                                                           dfb, f_in, unit, e1_io, e2bar, ubar); NN_LAUNCHED(1);
     }
     NN_CHECK_LAUNCH("pair_bwd_gather");
     return 0;
@@ -890,10 +878,10 @@ int nn_node_aggregate_bwd_launch(const nn_nbr* nl, int n_rows, const float* t, c
     if (N <= 0) return 0;
     int grid = nn_ceil_div(N, kAggWarps);
     if (first) {
-        nn_launch_dep(k_node_aggregate_bwd<true>, dim3(grid), dim3(kAggThreads), 0, s, nl->status, nl->row_ptr, nl->col, nl->edge_pair, N, t, mn, e2, dfb, mnbar, fbar_new); NN_LAUNCHED(1);
+        k_node_aggregate_bwd<true><<<grid, kAggThreads, 0, s>>>(nl->status, nl->row_ptr, nl->col, nl->edge_pair, N, t, mn, e2, dfb, mnbar, fbar_new); NN_LAUNCHED(1);
     }
     else {
-        nn_launch_dep(k_node_aggregate_bwd<false>, dim3(grid), dim3(kAggThreads), 0, s, nl->status, nl->row_ptr, nl->col, nl->edge_pair, N, t, mn, e2, dfb, mnbar, fbar_new); NN_LAUNCHED(1);
+        k_node_aggregate_bwd<false><<<grid, kAggThreads, 0, s>>>(nl->status, nl->row_ptr, nl->col, nl->edge_pair, N, t, mn, e2, dfb, mnbar, fbar_new); NN_LAUNCHED(1);
     }
     NN_CHECK_LAUNCH("node_aggregate_bwd");
     return 0;

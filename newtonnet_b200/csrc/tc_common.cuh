@@ -1,5 +1,6 @@
-// PTX helpers shared by the tcgen05 kernels (gemm_tc.cu, message_tc.cu): mbarriers, bulk async copies,
-// UMMA descriptors, tcgen05.mma / commit / ld, the K-major 128B swizzle, the tf32 hi/lo split.
+// Helpers shared by the tcgen05 kernels (gemm_tc.cu, gemm_ts.cu, gemm_chain.cu, gemm_tn_tc.cu, message_tc.cu): mbarriers,
+// bulk async copies, UMMA descriptors, tcgen05.mma / commit / ld / st, the K-major 128B swizzle, the tf32 hi/lo split, the
+// MMA issue of one TS-mode tile, PDL, and the nn_gemm128 prologues / epilogues of the SS- and TS-mode backends.
 #pragma once
 #include "common.cuh"
 
@@ -9,6 +10,7 @@ constexpr int TM = 128;                       // rows per tile (UMMA M)
 constexpr int KB = 32;                        // K elements per swizzle atom row (128 B)
 constexpr uint32_t BLK_BYTES = TM * KB * 4;   // one [128 x 32] fp32 block = 16 KB
 constexpr uint32_t STG_BYTES = 32 * 32 * 4;   // per epilogue warp: one 32 x 32 fp32 chunk, XOR-swizzled
+constexpr int NKB = 4;                        // K blocks of a 128 x 128 contraction (K = 128)
 
 // instruction descriptor (cute::UMMA::InstrDescriptor): D=f32 (bits 4-5 = 1), A=B=tf32 (bits 7-9, 10-12
 // = 2), both K-major (bits 15,16 = 0), N>>3 at bits 17-22, M>>4 at bits 24-28.
@@ -111,6 +113,69 @@ __device__ __forceinline__ float tf32_hi(float x) {
     uint32_t u;
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(x));
     return __uint_as_float(u);
+}
+
+// MMAs of one 128 x 128 accumulator tile at d_tmem in TS mode.  K block kb of A is the hi / lo pair of 32-column groups at
+// a_tmem + 64 kb in tensor memory, B the resident image at sB ([hi|lo][kb][16 KB]).  Each K block waits for its producers
+// (bar_a_full[kb], parity `phase`) and is handed back to them (bar_a_empty[kb]) when its MMAs retire.
+__device__ __forceinline__ void umma_tile_ts(uint32_t d_tmem, uint32_t a_tmem, uint32_t sB, uint32_t bar_a_full,
+                                             uint32_t bar_a_empty, uint32_t phase) {
+    for (int kb = 0; kb < NKB; ++kb) {
+        mbar_wait(bar_a_full + 8 * kb, phase);
+        tc_fence_after();
+        const uint32_t a_hi = a_tmem + kb * 64, a_lo = a_hi + 32;
+        const uint32_t b_hi = sB + kb * BLK_BYTES, b_lo = b_hi + NKB * BLK_BYTES;
+#pragma unroll
+        for (int ks = 0; ks < KB / 8; ++ks) {                  // UMMA_K = 8 tf32 = 8 TMEM columns / 32 bytes
+            const uint64_t dbh = make_desc(b_hi + ks * 32), dbl = make_desc(b_lo + ks * 32);
+            umma_tf32_ts(d_tmem, a_lo + ks * 8, dbh, (kb | ks) != 0);   // small terms first
+            umma_tf32_ts(d_tmem, a_hi + ks * 8, dbl, 1);
+            umma_tf32_ts(d_tmem, a_hi + ks * 8, dbh, 1);
+        }
+        umma_commit(bar_a_empty + 8 * kb);                     // K block's TMEM columns reusable
+    }
+}
+
+// ---- nn_gemm128 prologues and epilogues (gemm_tc.cu, gemm_ts.cu) ---------------------------------------------------
+// Loads are issued raw (so they stay in flight); the prologue is applied when the value is consumed.
+template <int PRO>
+__device__ __forceinline__ float4 load_a(const nn_gemm_args& a, int grow, int k, int M) {
+    if (grow >= M) return f4_zero();
+    float4 v = ld4(a.X + (size_t)grow * 128 + k);
+    if (PRO == NN_PRO_ROWSCALE3) v = f4_mul(v, ld4(a.aux2 + (size_t)(grow / 3) * 128 + k));
+    return v;
+}
+template <int PRO>
+__device__ __forceinline__ float4 apply_prologue(const nn_gemm_args& a, float4 v, int grow, int k, int M) {
+    if (PRO == NN_PRO_SILU) { v.x = silu_f(v.x); v.y = silu_f(v.y); v.z = silu_f(v.z); v.w = silu_f(v.w); }
+    if (PRO == NN_PRO_SILU_SAVE) {
+        // one sigmoid per element serves silu (this product) and silu' (kept for the reverse sweep)
+        const float4 s = make_float4(sigmoid_f(v.x), sigmoid_f(v.y), sigmoid_f(v.z), sigmoid_f(v.w));
+        if (grow < M)
+            st4(a.aux_out + (size_t)grow * 128 + k,
+                make_float4(s.x * fmaf(v.x, 1.0f - s.x, 1.0f), s.y * fmaf(v.y, 1.0f - s.y, 1.0f),
+                            s.z * fmaf(v.z, 1.0f - s.z, 1.0f), s.w * fmaf(v.w, 1.0f - s.w, 1.0f)));
+        v = f4_mul(v, s);
+    }
+    return v;
+}
+
+template <int EPI>
+__device__ __forceinline__ float4 epilogue(const nn_gemm_args& a, float4 acc, int grow, int col) {
+    if (EPI == NN_EPI_BIAS) {
+        if (a.bias) acc = f4_add(acc, ld4(a.bias + col));
+    } else if (EPI == NN_EPI_DSILU) {
+        float4 p = ld4(a.aux1 + (size_t)grow * 128 + col);
+        acc.x *= dsilu_f(p.x); acc.y *= dsilu_f(p.y); acc.z *= dsilu_f(p.z); acc.w *= dsilu_f(p.w);
+    } else if (EPI == NN_EPI_ADD) {
+        acc = f4_add(acc, ld4(a.aux1 + (size_t)grow * 128 + col));
+    } else if (EPI == NN_EPI_EQUIV_BWD) {
+        float4 fb = ld4(a.aux1 + (size_t)grow * 128 + col);
+        float4 ab = ld4(a.aux2 + (size_t)(grow / 3) * 128 + col);
+        float4 g = ld4(a.aux3 + (size_t)grow * 128 + col);
+        acc = f4_add(acc, f4_fma(ab, g, fb));
+    }
+    return acc;
 }
 
 // ---- programmatic dependent launch (PDL) ------------------------------------------------------------------

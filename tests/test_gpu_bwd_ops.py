@@ -69,7 +69,7 @@ def test_mlp_fwd_bwd(M, pair_level):
     gX, = torch.autograd.grad(want, Xd, G.double())
     for accumulate in (0, 1):
         out = acc0.clone()
-        tmp = torch.empty(Mp, 128, device=DEV)
+        tmp = torch.empty_like(X)
         L.check(lib.nn_mlp_bwd(G.data_ptr(), C.byref(M2), mid.data_ptr(), tmp.data_ptr(), C.byref(M1), out.data_ptr(), M, L.ptr(cnt),
                                accumulate, s), 'nn_mlp_bwd')
         torch.testing.assert_close(out.double(), gX + (acc0.double() if accumulate else 0), **TOL)

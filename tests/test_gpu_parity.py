@@ -108,7 +108,8 @@ def test_neighbor_list_errors():
 
 
 # ----------------------------------------------------------------------------- dense contraction
-def _gemm(lib, X, B, pro=0, epi=0, bias=None, aux1=None, aux2=None, aux3=None, m_dev=None, mul=1, Y=None, aux_out=None):
+def _gemm(lib, X, B, pro=0, epi=0, bias=None, aux1=None, aux2=None, aux3=None, m_dev=None, mul=1, Y=None, aux_out=None,
+          aux_tiled=0):
     from newtonnet_b200 import _lib as L
     a = L.GemmArgs()
     Y = torch.empty_like(X) if Y is None else Y
@@ -116,7 +117,7 @@ def _gemm(lib, X, B, pro=0, epi=0, bias=None, aux1=None, aux2=None, aux3=None, m
     L.check(lib.nn_gemm128_prepare_b(B.data_ptr(), img.data_ptr(), torch.cuda.current_stream().cuda_stream), 'prepare_b')
     a.X, a.B, a.B_img, a.Y = X.data_ptr(), B.data_ptr(), img.data_ptr(), Y.data_ptr()
     a.bias, a.aux1, a.aux2, a.aux3, a.aux_out = L.ptr(bias), L.ptr(aux1), L.ptr(aux2), L.ptr(aux3), L.ptr(aux_out)
-    a.m_dev, a.m_dev_mul, a.m, a.prologue, a.epilogue = L.ptr(m_dev), mul, X.shape[0], pro, epi
+    a.m_dev, a.m_dev_mul, a.m, a.prologue, a.epilogue, a.aux_tiled = L.ptr(m_dev), mul, X.shape[0], pro, epi, aux_tiled
     L.check(lib.nn_gemm128(C.byref(a), torch.cuda.current_stream().cuda_stream), 'nn_gemm128')
     return Y
 

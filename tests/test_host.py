@@ -32,7 +32,7 @@ def test_library_loads_and_exports_every_declared_symbol():
     assert C.sizeof(_lib.LayerWeights) == 7 * 32 + 7 * 8
     assert C.sizeof(_lib.Weights) == 8 + 2 * 8 + 8 * (7 * 32 + 7 * 8) + 2 * 32 + 6 * 8 + 3 * 32 + 4 * 8
     assert C.sizeof(_lib.Nbr) == 6 * 4 + 13 * 8 + 8
-    assert C.sizeof(_lib.GemmArgs) == 10 * 8 + 6 * 4
+    assert C.sizeof(_lib.GemmArgs) == 10 * 8 + 5 * 4 + 4       # five int32 fields, padded to pointer alignment
     assert lib.nn_nbr_workspace_bytes(1000, 4) > 0
     assert lib.nn_eval_workspace_bytes(1000, 4, 30000, 3, 1) > lib.nn_eval_workspace_bytes(1000, 4, 30000, 3, 0)
 
